@@ -1,7 +1,7 @@
 """bench.py -- headline benchmark: Van der Pol ensemble of 65,536 randomised initial conditions.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--members B]
-                    [--workload vdp|c4] [--scaling weak|strong]
+                    [--workload vdp|c4] [--scaling weak|strong] [--dump-outputs DIR]
 
 Workload `vdp` (default; BASELINE.json configs[1], SURVEY 8d C2): stiff Van der Pol (mu=1e3), dense EKF1
 (ode_order=2) + fixed-point smoother at 50 checkpoints on [0, 6.3], nu=4, dynamic calibration,
@@ -26,6 +26,11 @@ fp64-CUDA-core bound, not HBM or tensor bound -- `roofline.hbm` shows the HBM si
 installed here) on the host cores on a bounded sample of the same members -- whose results are also
 compared with the GPU's for those members, bit for bit (`parity_checked_members`): the bench fails if
 they differ.
+
+`--dump-outputs DIR` writes what the last timed step returned, so that two builds can be compared output
+for output on identical seeded inputs: DIR/members.npy (global member indices) and DIR/nu<nu>_<key>.npy
+for key in u, u_std, n_accepted, n_rejected, status (float64; the counters are exact), rows in member
+order.  When all members would exceed DUMP_BYTES, a fixed seeded sample of members is written.
 """
 
 import argparse
@@ -55,6 +60,8 @@ NU = 4
 METRIC = "ivp_solves_per_s"
 UNIT = "IVP-solves/s"
 PARITY_TOL = 1e-9  # north_star: checkpoint means / standard deviations within 1e-9 relative
+DUMP_BYTES = 32 << 20  # --dump-outputs writes at most this much
+DUMP_KEYS = ("u", "u_std", "n_accepted", "n_rejected", "status")
 
 
 def flops_dense_fixedpoint(n, d, f_vf, f_jac):
@@ -296,6 +303,27 @@ def cpu_oracle_run(wl, first, count, threads):
     return secs, acc, outs
 
 
+def dump_outputs(path, nus, results, first=0):
+    """--dump-outputs: results[i] = {key: [B, ...] numpy array or torch tensor} of the launch with nu = nus[i], row r
+    being member first + r of the seeded ensemble.  All rows, or a fixed seeded sample of them that fits DUMP_BYTES."""
+    B = len(results[0]["u"])
+    per_member = 8 + sum(8 * int(np.prod(res[k].shape[1:])) for res in results for k in DUMP_KEYS)
+    n = min(B, DUMP_BYTES // per_member)
+    rows = np.arange(B) if n == B else np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "members.npy"), (first + rows).astype(np.float64))
+    for nu, res in zip(nus, results):
+        for k in DUMP_KEYS:
+            x = res[k]
+            if isinstance(x, np.ndarray):
+                x = x[rows]
+            else:
+                import torch
+
+                x = x[torch.from_numpy(rows).to(x.device)].cpu().numpy()
+            np.save(os.path.join(path, f"nu{nu}_{k}.npy"), x.astype(np.float64))
+
+
 def parity_against(outs_cpu, outs_gpu):
     """Compares oracle and GPU results member by member.  Returns (max relative difference of u / u_std,
     bit-exact?, counts identical?)."""
@@ -332,10 +360,12 @@ def run_reference(args):
     done, secs, acc = 0, 0.0, 0.0
     for i in range(args.steps):
         first = (i * chunk) % max(1, sample - chunk + 1) if sample > chunk else 0
-        s, a, _ = cpu_oracle_run(wl, first, min(chunk, sample), cores)
+        s, a, outs = cpu_oracle_run(wl, first, min(chunk, sample), cores)
         secs += s
         acc += a
         done += min(chunk, sample) * len(wl.nus)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, wl.nus, outs, first)
     value = done / secs
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -375,7 +405,10 @@ def main():
     ap.add_argument("--members", type=int, default=0, help="members per GPU (weak) / in total (strong); default: the workload's")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-strong", action="store_true", help="N>1: skip the additional strong-scaling measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -411,8 +444,9 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    def measure(scaling, steps, warmup, sample_clocks):
-        """Times `steps` passes over the ensemble.  weak: `members` per rank; strong: `members` in total."""
+    def measure(scaling, steps, warmup, sample_clocks, dump_dir=None):
+        """Times `steps` passes over the ensemble.  weak: `members` per rank; strong: `members` in total.
+        dump_dir: where rank 0 writes the results of the last timed step (--dump-outputs)."""
         B_total = members * world if scaling == "weak" else members
         sizes = ensemble.shard_sizes(B_total, world)
         B = sizes[rank]
@@ -450,6 +484,10 @@ def main():
         barrier()
         elapsed_ms = e0.elapsed_time(e1)
         clocks = sampler.stop() if sampler else None
+        if dump_dir and rank == 0:  # before the pass below overwrites the outputs
+            res = [L["out"] if world == 1 else {k: L["packed"].member_order(v) for k, v in L["gathered"].items()}
+                   for L in launches]  # fmt: skip
+            dump_outputs(dump_dir, wl.nus, res)
         # kernel times of one more (untimed) pass, launch by launch, from events on the launching stream
         kernel_ms, smooth_ms = [], []
         flush.zero_()
@@ -481,7 +519,7 @@ def main():
         }  # fmt: skip
 
     fp64_peak = _cabi.measure_fp64_peak()
-    head = measure(args.scaling, args.steps, args.warmup, True)
+    head = measure(args.scaling, args.steps, args.warmup, True, args.dump_outputs)
     other = None
     if world > 1 and not args.no_strong:
         other = measure("strong" if args.scaling == "weak" else "weak", args.steps, args.warmup, False)

@@ -5,9 +5,12 @@ import this module.  See oracle/pn_oracle.h for what the oracle restates and how
 it is pinned against the reference's golden artefacts.
 """
 
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -64,14 +67,21 @@ class AttemptInfo(C.Structure):
 
 
 def build(force=False):
-    """Compile oracle/libpn_oracle.so with gcc (see oracle/Makefile)."""
+    """Compile oracle/libpn_oracle.so with gcc (see oracle/Makefile) and return its path.  In a read-only
+    tree whose library is missing or older than its sources, the library is built in a temporary directory
+    (removed at exit) instead, so that running the tests or the benchmark never writes into the tree."""
     srcs = ["pn_linalg.c", "pn_blocked.c", "pn_problems.c", "pn_solver.c", "pn_oracle.h", "pn_internal.h", "Makefile"]
     if not force and os.path.exists(_LIB_PATH):
         newest = max(os.path.getmtime(os.path.join(_HERE, s)) for s in srcs)
         if os.path.getmtime(_LIB_PATH) >= newest:
             return _LIB_PATH
-    subprocess.run(["make", "-C", _HERE, "-B", "libpn_oracle.so"], check=True, capture_output=True)
-    return _LIB_PATH
+    out = _LIB_PATH
+    if not os.access(_HERE, os.W_OK):
+        tmp = tempfile.mkdtemp(prefix="pn_oracle_")
+        atexit.register(shutil.rmtree, tmp, True)
+        out = os.path.join(tmp, "libpn_oracle.so")
+    subprocess.run(["make", "-C", _HERE, "-B", f"LIB={out}"], check=True, capture_output=True)
+    return out
 
 
 _lib = None
@@ -80,8 +90,7 @@ _lib = None
 def lib():
     global _lib
     if _lib is None:
-        build()
-        _lib = C.CDLL(_LIB_PATH)
+        _lib = C.CDLL(build())
         dp = C.POINTER(C.c_double)
         _lib.pn_det_pow.restype = C.c_double
         _lib.pn_det_pow.argtypes = [C.c_double, C.c_double]

@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 pytestmark = pytest.mark.gpu
@@ -41,3 +42,24 @@ def test_one_json_line_with_the_contract_keys():
     assert roof["bound"] == "fp64" and roof["unit"] == "TFLOP/s"
     assert abs(roof["frac"] - roof["achieved"] / roof["peak"]) < 1e-12 and 0.0 < roof["frac"] < 1.0
     assert {"sm_mhz", "sm_max_mhz", "reasons"} <= set(line["clocks"])
+
+
+def test_dump_outputs_repeat_across_runs_and_match_the_reference_arm(tmp_path):
+    """--dump-outputs: float64 arrays of at most 64 MB in all; the seeded inputs make two runs with different step
+    counts write identical outputs, and the members both arms computed are bit-identical to the reference arm's."""
+    dirs = [tmp_path / n for n in ("a", "b", "ref")]
+    line = _run("--steps", "1", "--warmup", "0", "--members", "4096", "--no-cpu-baseline", "--dump-outputs", str(dirs[0]))
+    assert line["steps"] == 1
+    _run("--steps", "3", "--warmup", "0", "--members", "4096", "--no-cpu-baseline", "--dump-outputs", str(dirs[1]))
+    _run("--impl", "reference", "--steps", "1", "--warmup", "0", "--members", "64", "--dump-outputs", str(dirs[2]))
+    names = sorted(p.name for p in dirs[0].iterdir())
+    assert names == sorted(p.name for p in dirs[2].iterdir())
+    assert sum(p.stat().st_size for p in dirs[0].iterdir()) <= 64 << 20
+    a, b, ref = ({p.stem: np.load(p) for p in d.iterdir()} for d in dirs)
+    assert np.array_equal(a["members"], np.arange(4096)) and a["nu4_u"].shape == (4096, 50, 1)
+    assert (a["nu4_status"] == 0).all()
+    rows = ref["members"].astype(np.int64)
+    assert len(rows) > 0
+    for k in a:
+        assert a[k].dtype == np.float64 and np.array_equal(a[k], b[k], equal_nan=True), k
+        assert np.array_equal(a[k][rows], ref[k], equal_nan=True), k

@@ -211,3 +211,39 @@ def test_reference_arm_prints_one_json_line_with_the_contract_keys():
     r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0"],
                        capture_output=True, text=True, env=env, timeout=600)  # fmt: skip
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+def test_reference_arm_dumps_the_last_step_outputs(tmp_path, oracle):
+    """`--dump-outputs DIR` writes the results of the last timed step as float64 .npy files: the oracle's results for
+    the seeded members it names."""
+    import subprocess
+    import sys
+
+    import bench
+
+    env = {k: v for k, v in os.environ.items() if k not in ("RANK", "LOCAL_RANK", "WORLD_SIZE")}
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2", "--warmup", "0",
+                        "--members", "16", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, env=env,
+                       timeout=600)  # fmt: skip
+    assert r.returncode == 0, r.stderr[-2000:]
+    keys = ("u", "u_std", "n_accepted", "n_rejected", "status")
+    assert sorted(p.name for p in tmp_path.iterdir()) == sorted(["members.npy"] + [f"nu4_{k}.npy" for k in keys])
+    got = {p.stem: np.load(p) for p in tmp_path.iterdir()}
+    assert all(x.dtype == np.float64 for x in got.values())
+    members = got["members"].astype(np.int64)
+    assert len(members) > 0 and np.array_equal(members, members[0] + np.arange(len(members)))
+    u0, par = bench.ensemble_inputs(int(members[0]), len(members))
+    cfg = oracle.make_config("van_der_pol", 1, 4, 2, factorisation="dense", correction="ts1", strategy="fixedpoint",
+                             calibration="dynamic", atol=1e-6, rtol=1e-6, dt0=0.01, num_params=1)  # fmt: skip
+    want = oracle.solve_save_at_batch(cfg, u0, par, np.linspace(0.0, 6.3, 50))
+    for k in keys:
+        assert np.array_equal(got[f"nu4_{k}"], want[k].astype(np.float64)), k
+
+
+def test_bench_rejects_zero_steps():
+    import subprocess
+    import sys
+
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"],
+                       capture_output=True, text=True, timeout=600)  # fmt: skip
+    assert r.returncode != 0 and "--steps" in r.stderr
