@@ -177,9 +177,8 @@ __global__ void pn_order_scatter_kernel(const double* tol, long long B, unsigned
   if (i < B) order[atomicAdd(&cursor[order_bucket(tol[2 * i], tol[2 * i + 1])], 1u)] = i;
 }
 
-constexpr long long PAIR_MAX_BATCH = 148 * 128;  // thread-per-IVP PAIR build: one 128-lane CTA per SM
+constexpr long long PAIR_MAX_MEMBERS = 148 * 128;  // thread-per-IVP PAIR build: one 128-lane CTA per SM
 constexpr long long WIDE_WARP_MIN_BATCH = 592;  // CTA-per-IVP isotropic family: one warp per IVP from four members per SM on
-constexpr long long COOP_MAX_BATCH = 0;        // largest ensemble the cooperative scalar kernel is chosen for (0: opt-in only)
 constexpr long long DENSE_CTA_MAX_CTAS = 296;  // per-CTA scratch regions the workspace provides (2 per SM of a B200)
 static size_t dense_cta_smem_bytes(const KernelEntry* k, const pn_b200_desc* d) {
   const int Dn = (d->nu + 1) * d->d;
@@ -204,29 +203,13 @@ static int resolve(const pn_b200_desc* d, const KernelEntry** out) {
                    (d->factorisation == PN_B200_DENSE && d->d == 1) ||
                    (d->factorisation == PN_B200_BLOCKDIAG && d->d == 1 && d->correction == PN_B200_TS0);
   if (scalar_ok) k = find_kernel(FAMILY_SCALAR, d->problem, d->nu, d->strategy, d->d);
-  // Scalar ODEs, n lanes per IVP instead of one (pn_coop_kernel.cuh): opt-in.  Measured on B200 (profiles/
-  // r02_small_ensembles.txt): one attempted step is a ~5k-cycle chain of dependent fp64 operations (12 serial
-  // reflectors + the controller's log / exp), which neither mapping can shorten; spreading the columns over
-  // n lanes removes arithmetic from the lanes but adds exchanges to the chain, and ends up 15-60 % SLOWER than
-  // the thread-per-IVP kernel at every ensemble size (1 member: 81 vs 70 ms; 8,192: 126 vs 78 ms).  It stays
-  // in the tree as a bit-identical cross-check and for experiments: PN_B200_COOP_MAX_BATCH=<members>.
-  if (k && d->d == 1 && d->calibration != PN_B200_CALIB_MLE && !getenv("PN_B200_NO_COOP")) {
-    long long coop_max = COOP_MAX_BATCH;
-    if (const char* e = getenv("PN_B200_COOP_MAX_BATCH")) coop_max = atoll(e);
-    if (d->batch <= coop_max) {
-      const KernelEntry* kc = find_kernel(FAMILY_COOP, d->problem, d->nu, d->strategy, d->d);
-      if (kc) k = kc;
-    }
-  }
   // Small ensembles of the thread-per-IVP family, fixed-point strategy: filter lane + backward lane per IVP
-  // (PAIR build) while the members fit one filter warp per SM sub-partition (PN_B200_PAIR=0 switches it off,
-  // PN_B200_PAIR_MAX_BATCH=<members> moves the limit; results are bit-identical either way)
+  // (PAIR build) while the members fit one filter warp per SM sub-partition (PN_B200_PAIR=0 switches it off;
+  // results are bit-identical either way)
   if (k && k->family == FAMILY_SCALAR && d->strategy == PN_B200_FIXEDPOINT && d->calibration != PN_B200_CALIB_MLE &&
       !(d->flags & PN_B200_FLAG_RECORD)) {
     const char* pe = getenv("PN_B200_PAIR");
-    long long pair_max = PAIR_MAX_BATCH;
-    if (const char* e = getenv("PN_B200_PAIR_MAX_BATCH")) pair_max = atoll(e);
-    if (!(pe && pe[0] == '0') && d->batch <= pair_max) {
+    if (!(pe && pe[0] == '0') && d->batch <= PAIR_MAX_MEMBERS) {
       const KernelEntry* kp = find_kernel(FAMILY_PAIR, d->problem, d->nu, d->strategy, d->d);
       if (kp) k = kp;
     }
@@ -236,11 +219,10 @@ static int resolve(const pn_b200_desc* d, const KernelEntry** out) {
     k = find_kernel(FAMILY_GROUP_BDIAG, d->problem, d->nu, d->strategy, d->d);
   if (!k && d->correction == PN_B200_TS0 && d->factorisation == PN_B200_ISOTROPIC)
     k = find_kernel(FAMILY_GROUP_ISO, d->problem, d->nu, d->strategy, d->d);
-  // warp-per-IVP dense family: dense factorisation with d > 1, EKF0 or EKF1
+  // warp-per-IVP dense family: dense factorisation with d > 1, EKF0 or EKF1; the register-column kernel (D <= 32),
+  // else the shared-memory kernel
   if (!k && d->factorisation == PN_B200_DENSE && d->d > 1) {
-    // register-column kernel first (D <= 32); PN_B200_DENSE_SMEM=1 forces the shared-memory kernel (A/B runs)
-    const char* force = getenv("PN_B200_DENSE_SMEM");
-    if (!(force && force[0] == '1')) k = find_kernel(FAMILY_DENSE_ROWS, d->problem, d->nu, d->strategy, d->d);
+    k = find_kernel(FAMILY_DENSE_ROWS, d->problem, d->nu, d->strategy, d->d);
     if (!k) k = find_kernel(FAMILY_DENSE, d->problem, d->nu, d->strategy, d->d);
   }
   // CTA-per-IVP dense family: dense factorisation with a large runtime dimension (Brusselator N >= 5:
@@ -249,7 +231,7 @@ static int resolve(const pn_b200_desc* d, const KernelEntry** out) {
     k = find_kernel(FAMILY_DENSE_CTA, d->problem, d->nu, d->strategy, 0);
     if (k && dense_cta_smem_bytes(k, d) > WIDE_SMEM_LIMIT_BYTES) k = nullptr;  // D too large for one CTA's panel
     // two CTAs per SM when their shared memory fits (+1 KB reserved per CTA) and there are members for them
-    if (k && 2 * (dense_cta_smem_bytes(k, d) + 1024) <= WIDE_SMEM_LIMIT_BYTES && d->batch > 148 && !getenv("PN_B200_DENSE_CTA_ONE")) {
+    if (k && 2 * (dense_cta_smem_bytes(k, d) + 1024) <= WIDE_SMEM_LIMIT_BYTES && d->batch > 148) {
       const KernelEntry* k2 = find_kernel(FAMILY_DENSE_CTA, d->problem, d->nu, d->strategy, -2);
       if (k2) k = k2;
     }
@@ -274,8 +256,8 @@ static int resolve(const pn_b200_desc* d, const KernelEntry** out) {
       }
     }
   }
-  if (k && (d->flags & PN_B200_FLAG_RECORD) && k->family != FAMILY_SCALAR && k->family != FAMILY_COOP &&
-      k->family != FAMILY_GROUP_ISO && k->family != FAMILY_GROUP_BDIAG && k->family != FAMILY_WIDE)
+  if (k && (d->flags & PN_B200_FLAG_RECORD) && k->family != FAMILY_SCALAR && k->family != FAMILY_GROUP_ISO &&
+      k->family != FAMILY_GROUP_BDIAG && k->family != FAMILY_WIDE)
     return fail(PN_B200_ERR_UNSUPPORTED, "trajectory recording is implemented for the thread-per-IVP, lane-per-dimension and CTA-per-IVP isotropic kernels");
   if (!k) {
     char buf[256];
@@ -299,12 +281,11 @@ static int make_plan(const pn_b200_desc* d, Plan* p, bool need_device) {
                 ? (size_t)p->k->smem_doubles * (p->k->threads / 32) * sizeof(double)  // per warp
                 : (size_t)p->k->smem_doubles * p->k->threads * sizeof(double);        // per thread
   if (p->k->family == FAMILY_DENSE_CTA) p->smem = dense_cta_smem_bytes(p->k, d);
-  if (p->k->family == FAMILY_COOP) p->smem = (size_t)p->k->smem_doubles * sizeof(double);  // per CTA
   if (p->k->family == FAMILY_WIDE) {
     p->smem += ((size_t)2 * d->d + p->k->threads / 32 + 2) * sizeof(double);
     // few members (at most one per SM: no occupancy to lose) whose mean arrays fit next to the rest
     const size_t one = (size_t)(d->nu + 1) * d->d * sizeof(double);
-    if (d->batch <= WIDE_SMEM_MAX_MEMBERS && !getenv("PN_B200_WIDE_GLOBAL_MEANS")) {
+    if (d->batch <= WIDE_SMEM_MAX_MEMBERS) {
       while (p->wide_smem_means < 3 && p->smem + one <= WIDE_SMEM_LIMIT_BYTES) {
         p->smem += one;
         p->wide_smem_means += 1;
@@ -377,7 +358,6 @@ static int make_plan(const pn_b200_desc* d, Plan* p, bool need_device) {
   }
   const int occ = p->ctas_per_sm;
   long long per_cta = (p->k->family == FAMILY_WIDE) ? 1 : p->k->threads / p->k->group;  // IVPs per CTA
-  if (p->k->family == FAMILY_COOP) per_cta = (long long)(p->k->threads / 32) * (32 / p->k->group);
   long long want = (d->batch + per_cta - 1) / per_cta;
   long long cap = (long long)occ * p->num_sms;
   if (p->k->family == FAMILY_DENSE_CTA && cap > DENSE_CTA_MAX_CTAS) cap = DENSE_CTA_MAX_CTAS;

@@ -1,8 +1,9 @@
 // pn_registry.h -- table of compiled kernel instances (one per problem functor x nu x strategy).
+// An entry names only kernels the library launches from it: what several builds share lives in *Slots helpers
+// that name no solve kernel, and each *Instance adds its own solve kernel(s).
 #pragma once
 #include <cuda_runtime.h>
 
-#include "pn_coop_kernel.cuh"
 #include "pn_dense_cta_kernel.cuh"
 #include "pn_dense_kernel.cuh"
 #include "pn_dense_rows_kernel.cuh"
@@ -21,7 +22,6 @@ enum : int {
   FAMILY_WIDE = 4,        // CTA per IVP, isotropic, runtime dimension (Brusselator d = 2N up to 4096)
   FAMILY_DENSE_ROWS = 5,  // 16 or 32 lanes per IVP, register-resident Householder columns (dense, D <= 32)
   FAMILY_DENSE_CTA = 6,   // CTA per IVP, dense with a large runtime dimension, blocked QR on the FP64 tensor path
-  FAMILY_COOP = 7,        // n lanes per IVP (scalar ODEs, small ensembles): columns of every QR spread over the lanes
   FAMILY_PAIR = 8         // thread per IVP + a backward lane per IVP in a partner warp (fixed-point, small ensembles)
 };
 inline bool family_is_dense(int family) { return family == FAMILY_DENSE || family == FAMILY_DENSE_ROWS; }
@@ -35,34 +35,27 @@ struct KernelEntry {
   int extra_threads = 0;  // threads of the CTA beyond `threads` that do not run the step (CTA-per-IVP PIPE build: the backward warp)
   int group;          // lanes per IVP (1: thread per IVP)
   int dv;             // lanes per IVP that own state (workspace entries per member)
-  int ctx_doubles;    // doubles one parked member occupies (time-sliced scheduling); 0: not supported
+  int ctx_doubles = 0;  // doubles one parked member occupies (time-sliced scheduling); 0: not supported
   bool has_jac;
   const void* solve_func;
-  const void* solve_func_sliced;  // time-sliced variant of the same kernel (nullptr: none)
+  const void* solve_func_sliced = nullptr;  // time-sliced variant of the same kernel (nullptr: none)
   cudaError_t (*launch_solve)(const SolveArgs&, int grid, size_t smem, cudaStream_t);
-  cudaError_t (*launch_solve_sliced)(const SolveArgs&, int grid, size_t smem, cudaStream_t);
+  cudaError_t (*launch_solve_sliced)(const SolveArgs&, int grid, size_t smem, cudaStream_t) = nullptr;
   cudaError_t (*launch_smooth)(const SmoothArgs&, cudaStream_t);
-  cudaError_t (*launch_sample)(const SampleArgs&, cudaStream_t);  // nullptr: family has no sampler yet
-  cudaError_t (*launch_lml)(const LmlArgs&, cudaStream_t);        // nullptr: no likelihood kernel for this family
+  cudaError_t (*launch_sample)(const SampleArgs&, cudaStream_t) = nullptr;  // nullptr: family has no sampler yet
+  cudaError_t (*launch_lml)(const LmlArgs&, cudaStream_t) = nullptr;        // nullptr: no likelihood kernel for this family
 };
 
 void register_kernel(const KernelEntry& e);
 const KernelEntry* find_kernel(int family, int problem, int nu, int strategy, int d);
 
-template <class Prob, int NU, int STRAT, int GROUP, int BDIAG, int THREADS>
-struct ScalarInstance {
+// what the thread-per-IVP and lane-per-dimension builds of one (problem, nu, strategy) share: slots, shared-memory
+// state, smoothing / sampling / likelihood kernels
+template <class Prob, int NU, int STRAT, int GROUP, int BDIAG>
+struct ScalarSlots {
   static constexpr int DL = (GROUP > 1) ? 1 : Prob::D;  // mean columns per lane
   static constexpr int DV = (GROUP > 1) ? Prob::D : 1;
-  static cudaError_t launch_solve(const SolveArgs& a, int grid, size_t smem, cudaStream_t s) {
-    pn_scalar_kernel<Prob, NU, STRAT, GROUP, BDIAG, THREADS><<<grid, THREADS, smem, s>>>(a);
-    return cudaGetLastError();
-  }
-  // time-sliced scheduling: compiled for the thread-per-IVP fixed-point kernels (the checkpoint solver)
-  static constexpr bool SLICED = (GROUP == 1 && STRAT == 1);
-  static cudaError_t launch_solve_sliced(const SolveArgs& a, int grid, size_t smem, cudaStream_t s) {
-    pn_scalar_kernel<Prob, NU, STRAT, GROUP, BDIAG, THREADS, 0, SLICED ? 1 : 0><<<grid, THREADS, smem, s>>>(a);
-    return cudaGetLastError();
-  }
+  using Lay = Layout<NU + 1, DL>;
   static cudaError_t launch_smooth(const SmoothArgs& a, cudaStream_t s) {
     int grid = (int)((a.B * a.dv + 127) / 128);
     pn_smooth_kernel<NU + 1, DL, STRAT><<<grid, 128, 0, s>>>(a);
@@ -79,7 +72,6 @@ struct ScalarInstance {
     return cudaGetLastError();
   }
   static KernelEntry entry() {
-    using Lay = Layout<NU + 1, DL>;
     KernelEntry e;
     e.launch_sample = (STRAT == 1) ? &launch_sample : nullptr;
     e.launch_lml = (STRAT == 1) ? &launch_lml : nullptr;
@@ -95,14 +87,35 @@ struct ScalarInstance {
     e.P = Prob::P;
     e.slot_doubles = (STRAT == 1) ? Lay::SLOT_FIX : Lay::SLOT_FILT;
     e.smem_doubles = ((STRAT == 1) ? Lay::BW : 0) + Lay::PEND + Lay::MARG;
-    e.ctx_doubles = SLICED ? slice_ctx_doubles(Lay::BW, Lay::MARG) : 0;
-    e.solve_func_sliced = SLICED ? (const void*)&pn_scalar_kernel<Prob, NU, STRAT, GROUP, BDIAG, THREADS, 0, SLICED ? 1 : 0> : nullptr;
-    e.launch_solve_sliced = SLICED ? &launch_solve_sliced : nullptr;
-    e.threads = THREADS;
     e.has_jac = Prob::HAS_JAC;
+    e.launch_smooth = &launch_smooth;
+    return e;
+  }
+};
+
+template <class Prob, int NU, int STRAT, int GROUP, int BDIAG, int THREADS>
+struct ScalarInstance {
+  using Slots = ScalarSlots<Prob, NU, STRAT, GROUP, BDIAG>;
+  static cudaError_t launch_solve(const SolveArgs& a, int grid, size_t smem, cudaStream_t s) {
+    pn_scalar_kernel<Prob, NU, STRAT, GROUP, BDIAG, THREADS><<<grid, THREADS, smem, s>>>(a);
+    return cudaGetLastError();
+  }
+  // time-sliced scheduling: compiled for the thread-per-IVP fixed-point kernels (the checkpoint solver)
+  static constexpr bool SLICED = (GROUP == 1 && STRAT == 1);
+  static cudaError_t launch_solve_sliced(const SolveArgs& a, int grid, size_t smem, cudaStream_t s) {
+    pn_scalar_kernel<Prob, NU, STRAT, GROUP, BDIAG, THREADS, 0, 1><<<grid, THREADS, smem, s>>>(a);
+    return cudaGetLastError();
+  }
+  static KernelEntry entry() {
+    KernelEntry e = Slots::entry();
+    e.threads = THREADS;
     e.solve_func = (const void*)&pn_scalar_kernel<Prob, NU, STRAT, GROUP, BDIAG, THREADS>;
     e.launch_solve = &launch_solve;
-    e.launch_smooth = &launch_smooth;
+    if constexpr (SLICED) {
+      e.ctx_doubles = slice_ctx_doubles(Slots::Lay::BW, Slots::Lay::MARG);
+      e.solve_func_sliced = (const void*)&pn_scalar_kernel<Prob, NU, STRAT, GROUP, BDIAG, THREADS, 0, 1>;
+      e.launch_solve_sliced = &launch_solve_sliced;
+    }
     return e;
   }
 };
@@ -124,14 +137,10 @@ inline cudaError_t launch_dense_sample(const SampleArgs& a, int Dn, int transpos
   return cudaGetLastError();
 }
 
-// dense factorisation with d > 1: warp per IVP
+// what the dense builds with d > 1 and WARPS warps per CTA share: slots, smoothing and sampling kernels
 template <class Prob, int NU, int STRAT, int WARPS>
-struct DenseInstance {
+struct DenseSlots {
   using Lay = DenseLayout<NU + 1, Prob::D>;
-  static cudaError_t launch_solve(const SolveArgs& a, int grid, size_t smem, cudaStream_t s) {
-    pn_dense_kernel<Prob, NU, STRAT, WARPS><<<grid, 32 * WARPS, smem, s>>>(a);
-    return cudaGetLastError();
-  }
   static cudaError_t launch_smooth(const SmoothArgs& a, cudaStream_t s) {
     const size_t smem = (size_t)WARPS * Lay::SMEM_SMOOTH * sizeof(double);
     auto kern = pn_dense_smooth_kernel<NU + 1, Prob::D, STRAT, WARPS>;
@@ -147,12 +156,6 @@ struct DenseInstance {
   static KernelEntry entry() {
     KernelEntry e;
     e.launch_sample = (STRAT == 1) ? &launch_sample : nullptr;
-    e.launch_lml = nullptr;
-    e.ctx_doubles = 0;
-    e.solve_func_sliced = nullptr;
-    e.launch_solve_sliced = nullptr;
-    e.family = FAMILY_DENSE;
-    e.group = 32;
     e.dv = 1;
     e.problem = Prob::ID;
     e.nu = NU;
@@ -162,12 +165,28 @@ struct DenseInstance {
     e.Q = Prob::Q;
     e.P = Prob::P;
     e.slot_doubles = (STRAT == 1) ? Lay::SLOT_FIX : Lay::SLOT_FILT;
-    e.smem_doubles = Lay::SMEM;  // per warp (= per 32 threads), see make_plan
     e.threads = 32 * WARPS;
     e.has_jac = Prob::HAS_JAC;
+    e.launch_smooth = &launch_smooth;
+    return e;
+  }
+};
+
+// dense factorisation with d > 1: warp per IVP, D x D factors in shared memory
+template <class Prob, int NU, int STRAT, int WARPS>
+struct DenseInstance {
+  using Slots = DenseSlots<Prob, NU, STRAT, WARPS>;
+  static cudaError_t launch_solve(const SolveArgs& a, int grid, size_t smem, cudaStream_t s) {
+    pn_dense_kernel<Prob, NU, STRAT, WARPS><<<grid, 32 * WARPS, smem, s>>>(a);
+    return cudaGetLastError();
+  }
+  static KernelEntry entry() {
+    KernelEntry e = Slots::entry();
+    e.family = FAMILY_DENSE;
+    e.group = 32;
+    e.smem_doubles = Slots::Lay::SMEM;  // per warp (= per 32 threads), see make_plan
     e.solve_func = (const void*)&pn_dense_kernel<Prob, NU, STRAT, WARPS>;
     e.launch_solve = &launch_solve;
-    e.launch_smooth = &launch_smooth;
     return e;
   }
 };
@@ -175,14 +194,13 @@ struct DenseInstance {
 // dense factorisation with d > 1 and D <= 32: LANES lanes per IVP, columns in registers
 template <class Prob, int NU, int STRAT, int LANES, int WARPS>
 struct DenseRowsInstance {
-  using Lay = DenseLayout<NU + 1, Prob::D>;
   using RL = DenseRowsLayout<NU + 1, Prob::D>;
   static cudaError_t launch_solve(const SolveArgs& a, int grid, size_t smem, cudaStream_t s) {
     pn_dense_rows_kernel<Prob, NU, STRAT, LANES, WARPS><<<grid, 32 * WARPS, smem, s>>>(a);
     return cudaGetLastError();
   }
   static KernelEntry entry() {
-    KernelEntry e = DenseInstance<Prob, NU, STRAT, WARPS>::entry();  // same slots, same smoothing kernel
+    KernelEntry e = DenseSlots<Prob, NU, STRAT, WARPS>::entry();
     e.family = FAMILY_DENSE_ROWS;
     e.group = LANES;
     e.smem_doubles = (32 / LANES) * RL::SMEM_SLOT + (RL::TABLES + WARPS - 1) / WARPS;  // per warp (the tables exist once per CTA), see make_plan
@@ -226,9 +244,6 @@ struct WideInstance {
     KernelEntry e;
     e.launch_sample = (STRAT == 1) ? &launch_sample : nullptr;
     e.launch_lml = (STRAT == 1) ? &launch_lml : nullptr;
-    e.ctx_doubles = 0;
-    e.solve_func_sliced = nullptr;
-    e.launch_solve_sliced = nullptr;
     e.family = FAMILY_WIDE;
     e.group = THREADS;
     e.dv = 1;
@@ -252,51 +267,21 @@ struct WideInstance {
   }
 };
 
-// scalar ODEs, small ensembles: n lanes per IVP (same slots / smoothing / sampling / likelihood kernels as the
-// thread-per-IVP family)
-template <class Prob, int NU, int STRAT, int THREADS>
-struct CoopInstance {
-  using Base = ScalarInstance<Prob, NU, STRAT, 1, 0, 128>;
-  static cudaError_t launch_solve(const SolveArgs& a, int grid, size_t smem, cudaStream_t s) {
-    pn_coop_kernel<Prob, NU, STRAT, THREADS><<<grid, THREADS, smem, s>>>(a);
-    return cudaGetLastError();
-  }
-  static KernelEntry entry() {
-    KernelEntry e = Base::entry();
-    using CL = CoopLayout<NU + 1>;
-    e.family = FAMILY_COOP;
-    e.group = NU + 1;
-    e.threads = THREADS;
-    e.smem_doubles = (THREADS / 32) * CL::G * CL::PER_GROUP + CL::STATE * THREADS;  // per CTA
-    e.ctx_doubles = 0;
-    e.solve_func_sliced = nullptr;
-    e.launch_solve_sliced = nullptr;
-    e.solve_func = (const void*)&pn_coop_kernel<Prob, NU, STRAT, THREADS>;
-    e.launch_solve = &launch_solve;
-    return e;
-  }
-};
-
 // thread-per-IVP kernels for small ensembles: THREADS filter lanes + THREADS backward lanes per CTA (PAIR = 1);
 // same slots / smoothing / sampling / likelihood kernels as the thread-per-IVP family
 template <class Prob, int NU, int THREADS>
 struct PairInstance {
-  using Base = ScalarInstance<Prob, NU, 1, 1, 0, 128>;
-  using Lay = Layout<NU + 1, Prob::D>;
   using MB = pair::Mailbox<NU + 1, Prob::D>;
   static cudaError_t launch_solve(const SolveArgs& a, int grid, size_t smem, cudaStream_t s) {
     pn_scalar_kernel<Prob, NU, 1, 1, 0, THREADS, 0, 0, 0, 1><<<grid, 2 * THREADS, smem, s>>>(a);
     return cudaGetLastError();
   }
   static KernelEntry entry() {
-    KernelEntry e = Base::entry();
+    KernelEntry e = ScalarSlots<Prob, NU, 1, 1, 0>::entry();
     e.family = FAMILY_PAIR;
     e.threads = THREADS;
     e.extra_threads = THREADS;
-    e.smem_doubles = Lay::BW + Lay::PEND + Lay::MARG + MB::DOUBLES + (MB::INTS + 1) / 2;  // per filter lane
-    e.ctx_doubles = 0;
-    e.solve_func_sliced = nullptr;
-    e.launch_solve_sliced = nullptr;
+    e.smem_doubles += MB::DOUBLES + (MB::INTS + 1) / 2;  // per filter lane: its thread-per-IVP state + the mailbox
     e.solve_func = (const void*)&pn_scalar_kernel<Prob, NU, 1, 1, 0, THREADS, 0, 0, 0, 1>;
     e.launch_solve = &launch_solve;
     return e;
@@ -328,10 +313,6 @@ struct DenseCtaInstance {
   static KernelEntry entry() {
     KernelEntry e;
     e.launch_sample = (STRAT == 1) ? &launch_sample : nullptr;
-    e.launch_lml = nullptr;
-    e.ctx_doubles = 0;
-    e.solve_func_sliced = nullptr;
-    e.launch_solve_sliced = nullptr;
     e.family = FAMILY_DENSE_CTA;
     e.group = cta::T;
     e.dv = 1;
@@ -370,8 +351,6 @@ struct Registrar {
   static ::pn::Registrar PN_CAT(pn_reg_, __COUNTER__)(::pn::DenseRowsInstance<::pn::Prob, NU, STRAT, LANES, WARPS>::entry())
 #define PN_REGISTER_PAIR(Prob, NU) \
   static ::pn::Registrar PN_CAT(pn_reg_, __COUNTER__)(::pn::PairInstance<::pn::Prob, NU, 128>::entry())
-#define PN_REGISTER_COOP(Prob, NU, STRAT) \
-  static ::pn::Registrar PN_CAT(pn_reg_, __COUNTER__)(::pn::CoopInstance<::pn::Prob, NU, STRAT, 128>::entry())
 #define PN_REGISTER_DENSE_CTA(Prob, NU, STRAT, NB, MINB) \
   static ::pn::Registrar PN_CAT(pn_reg_, __COUNTER__)(::pn::DenseCtaInstance<::pn::cta::Prob, NU, STRAT, NB, MINB>::entry())
 #define PN_REGISTER_WIDE(Prob, NU, STRAT) \

@@ -1,5 +1,5 @@
 """Small ensembles of the headline workload (VdP mu = 1e3, dense EKF1 + fixed-point, nu = 4, tol 1e-6, 50 checkpoints):
-ms per pass with and without the warp-by-warp member assignment (PN_B200_NO_PACK=1) and the PAIR build (PN_B200_PAIR=0).
+ms per pass with and without the PAIR build (PN_B200_PAIR=0).
 
     python scripts/small_ensemble_bench.py [members ...]      # on a B200
 """
@@ -19,10 +19,8 @@ for B in sizes:
     desc = _cabi.Desc(5, 1, 4, 2, 2, 1, 1, 1, 1e-6, 1e-6, 0.01, 0.95, 0.2, 10.0, 0.3, 0.4, B, K, 0, 1, 0, 0)
     u0_d = torch.as_tensor(u0, device=dev); par = torch.full((B, 1), 1e3, dtype=torch.float64, device=dev)
     save = torch.linspace(0, 6.3, K, dtype=torch.float64, device=dev)
-    for label, env in (("packed", {}), ("ticket", {"PN_B200_NO_PACK": "1"}), ("packed, no PAIR", {"PN_B200_PAIR": "0"}),
-                       ("ticket, no PAIR", {"PN_B200_PAIR": "0", "PN_B200_NO_PACK": "1"})):
-        for k in ("PN_B200_NO_PACK", "PN_B200_PAIR"):
-            os.environ.pop(k, None)
+    for label, env in (("PAIR", {}), ("no PAIR", {"PN_B200_PAIR": "0"})):
+        os.environ.pop("PN_B200_PAIR", None)
         os.environ.update(env)
         info = _cabi.kernel_info(desc)
         best, out = 1e30, None

@@ -8,13 +8,6 @@ import problems_util as pu
 pytestmark = pytest.mark.gpu
 
 
-@pytest.fixture(autouse=True)
-def _thread_per_ivp_kernels(monkeypatch):
-    """These tests pin the thread-per-IVP / lane-per-dimension kernels; the cooperative small-ensemble kernel
-    that would otherwise serve their d = 1 cases has its own module (tests/test_gpu_coop.py)."""
-    monkeypatch.setenv("PN_B200_NO_COOP", "1")
-
-
 def test_reference_test_case_logistic_checkpoint_solver():
     # tests/test_ivpsolvers.py:31-52 of the reference, with the closed form in place of diffrax
     from odecheckpts_b200 import ivps, ivpsolvers

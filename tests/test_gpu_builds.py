@@ -13,11 +13,6 @@ pytestmark = pytest.mark.gpu
 KEYS = ("u", "u_std", "marg_mean", "marg_chol", "n_accepted", "n_rejected", "status", "output_scale")
 
 
-@pytest.fixture(autouse=True)
-def _no_coop(monkeypatch):
-    monkeypatch.setenv("PN_B200_NO_COOP", "1")
-
-
 @pytest.mark.parametrize("B", [1, 33, 700])
 def test_pair_build_equals_the_plain_thread_per_ivp_kernel(cabi, oracle, monkeypatch, B):
     rng = np.random.default_rng(B)

@@ -1,6 +1,5 @@
-"""GPU parity tests of the cooperative scalar kernel (n lanes per IVP for d = 1 problems; opt-in through
-PN_B200_COOP_MAX_BATCH because it measured slower than the thread-per-IVP kernel, see DESIGN.md): bit for bit
-against the CPU oracle AND against the thread-per-IVP kernel."""
+"""Small ensembles of the d = 1 problems: the build the library picks (for the fixed-point strategy the PAIR build,
+a backward lane per IVP) bit for bit against the CPU oracle AND against the plain thread-per-IVP kernel."""
 
 import os
 
@@ -23,23 +22,18 @@ def cabi():
     return _cabi
 
 
-@pytest.fixture(autouse=True)
-def _enable_the_cooperative_kernel(monkeypatch):
-    monkeypatch.setenv("PN_B200_COOP_MAX_BATCH", "20000")
-
-
 class _thread_per_ivp:
-    """Forces the thread-per-IVP kernel for the calls inside (the library reads the variable per call)."""
+    """Forces the plain thread-per-IVP kernel for the calls inside (the library reads the variable per call)."""
 
     def __enter__(self):
-        self.old = os.environ.get("PN_B200_NO_COOP")
-        os.environ["PN_B200_NO_COOP"] = "1"
+        self.old = os.environ.get("PN_B200_PAIR")
+        os.environ["PN_B200_PAIR"] = "0"
 
     def __exit__(self, *exc):
         if self.old is None:
-            del os.environ["PN_B200_NO_COOP"]
+            del os.environ["PN_B200_PAIR"]
         else:
-            os.environ["PN_B200_NO_COOP"] = self.old
+            os.environ["PN_B200_PAIR"] = self.old
 
 
 def _desc(cabi, problem, nu, q, B, K, *, fact="dense", corr="ts1", strat="fixedpoint", calib="dynamic", atol=1e-6, rtol=1e-6,
@@ -66,15 +60,6 @@ def _vdp_members(B, seed=0):
     return u0, np.full((B, 1), 1e3)
 
 
-def test_the_cooperative_kernel_is_selected_for_small_ensembles_when_enabled(cabi):
-    info = cabi.kernel_info(_desc(cabi, "van_der_pol", 4, 2, 64, 10))
-    assert info["threads_per_cta"] == 128 and info["dynamic_smem_bytes"] < 60000  # exchange buffers + parked state
-    with _thread_per_ivp():
-        assert cabi.kernel_info(_desc(cabi, "van_der_pol", 4, 2, 64, 10))["dynamic_smem_bytes"] > 80000
-    # large ensembles keep the thread-per-IVP kernel
-    assert cabi.kernel_info(_desc(cabi, "van_der_pol", 4, 2, 65536, 10))["dynamic_smem_bytes"] > 80000
-
-
 @pytest.mark.parametrize("B,tol,strat,corr,calib,nu", [
     (1, 1e-3, "fixedpoint", "ts1", "dynamic", 4), (7, 1e-3, "fixedpoint", "ts1", "dynamic", 4), (64, 1e-6, "fixedpoint", "ts1", "dynamic", 4),
     (13, 1e-4, "filter", "ts1", "dynamic", 4), (9, 1e-4, "fixedpoint", "ts0", "none", 4), (11, 1e-3, "fixedpoint", "ts1", "dynamic", 2),
@@ -85,7 +70,7 @@ def test_van_der_pol_bitwise_against_the_oracle_and_the_thread_per_ivp_kernel(ca
     save_at = np.linspace(0.0, 6.3, K)
     kw = dict(corr=corr, strat=strat, calib=calib, atol=tol, rtol=tol)
     desc = _desc(cabi, "van_der_pol", nu, 2, B, K, **kw)
-    coop = cabi.solve_host(desc, u0, params, None, save_at, None, full=True)
+    got = cabi.solve_host(desc, u0, params, None, save_at, None, full=True)
     with _thread_per_ivp():
         ref = cabi.solve_host(desc, u0, params, None, save_at, None, full=True)
     cfg = oracle.make_config("van_der_pol", 1, nu, 2, factorisation="dense", correction=corr, strategy=strat, calibration=calib,
@@ -93,9 +78,9 @@ def test_van_der_pol_bitwise_against_the_oracle_and_the_thread_per_ivp_kernel(ca
     ora = oracle.solve_save_at_batch(cfg, u0, params, save_at)
     assert (ora["status"] == 0).all() and ora["n_accepted"][:, -1].min() > 100
     for key in ("status", "n_accepted", "n_rejected", "u", "u_std"):
-        _same(key + " (oracle)", coop[key], ora[key])
+        _same(key + " (oracle)", got[key], ora[key])
     for key in ("status", "n_accepted", "n_rejected", "u", "u_std", "marg_mean", "marg_chol", "output_scale"):
-        _same(key + " (thread-per-IVP kernel)", coop[key], ref[key])
+        _same(key + " (thread-per-IVP kernel)", got[key], ref[key])
 
 
 def test_per_member_tolerances_and_more_members_than_groups(cabi, oracle):
@@ -104,12 +89,16 @@ def test_per_member_tolerances_and_more_members_than_groups(cabi, oracle):
     tol = np.stack([10.0 ** -np.random.default_rng(1).integers(2, 5, B).astype(float)] * 2, 1)
     save_at = np.linspace(0.0, 1.0, K)
     desc = _desc(cabi, "van_der_pol", 4, 2, B, K)
-    coop = cabi.solve_host(desc, u0, params, tol, save_at, None)
+    got = cabi.solve_host(desc, u0, params, tol, save_at, None)
     with _thread_per_ivp():
         ref = cabi.solve_host(desc, u0, params, tol, save_at, None)
+    cfg = oracle.make_config("van_der_pol", 1, 4, 2, factorisation="dense", correction="ts1", atol=1e-6, rtol=1e-6,
+                             dt0=0.01, num_params=1)  # fmt: skip
+    ora = oracle.solve_save_at_batch(cfg, u0, params, save_at, tol=tol)
     for key in ("status", "n_accepted", "n_rejected", "u", "u_std"):
-        _same(key, coop[key], ref[key])
-    assert (coop["status"] == 0).all()
+        _same(key, got[key], ref[key])
+        _same(key + " (oracle)", got[key], ora[key])
+    assert (got["status"] == 0).all()
 
 
 def test_logistic_and_fixed_grid(cabi, oracle):
@@ -135,22 +124,22 @@ def test_logistic_and_fixed_grid(cabi, oracle):
 
 
 def test_save_every_step_recording(cabi, goldens):
-    """solve_adaptive_save_every_step (vdp.py:77-79) through the cooperative kernel: the recorded grid equals
-    the thread-per-IVP kernel's, and starts like the reference's golden grid."""
+    """solve_adaptive_save_every_step (vdp.py:77-79): the recorded grid is the same whichever thread-per-IVP build
+    runs, and starts like the reference's golden grid."""
     cap = 4096
     desc = _desc(cabi, "van_der_pol", 4, 2, 1, 2, strat="filter", atol=1e-3, rtol=1e-3, flags=cabi.FLAG_RECORD, cap=cap)
     args = (pu.van_der_pol_u0()[None], np.array([[1e3]]), None, np.array([0.0, 6.3]), None)
-    coop = cabi.solve_host(desc, *args)
+    got = cabi.solve_host(desc, *args)
     with _thread_per_ivp():
         ref = cabi.solve_host(desc, *args)
-    n = int(coop["traj_len"][0])
+    n = int(got["traj_len"][0])
     assert n == int(ref["traj_len"][0]) and 2800 < n < 3000
     for key in ("traj_t", "traj_u", "traj_std"):
-        _same(key, coop[key][:n], ref[key][:n])
-    np.testing.assert_allclose(coop["traj_t"][:20, 0], goldens["vdp_grid"][:20], rtol=1e-12)
+        _same(key, got[key][:n], ref[key][:n])
+    np.testing.assert_allclose(got["traj_t"][:20, 0], goldens["vdp_grid"][:20], rtol=1e-12)
 
 
-def test_sampling_and_likelihood_kernels_read_the_cooperative_kernels_workspace(cabi):
+def test_sampling_and_likelihood_kernels_read_the_pair_builds_workspace(cabi):
     import torch
 
     B, K = 5, 12

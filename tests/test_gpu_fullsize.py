@@ -7,13 +7,6 @@ import pytest
 pytestmark = pytest.mark.gpu
 
 
-@pytest.fixture(autouse=True)
-def _thread_per_ivp_kernels(monkeypatch):
-    """These tests pin the thread-per-IVP / lane-per-dimension kernels; the cooperative small-ensemble kernel
-    that would otherwise serve their d = 1 cases has its own module (tests/test_gpu_coop.py)."""
-    monkeypatch.setenv("PN_B200_NO_COOP", "1")
-
-
 @pytest.fixture(scope="module")
 def full_run():
     import torch

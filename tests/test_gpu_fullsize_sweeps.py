@@ -11,12 +11,6 @@ from test_gpu_parity import _assert_bitwise, _desc, _ocfg, cabi  # noqa: F401
 pytestmark = pytest.mark.gpu
 
 
-@pytest.fixture(autouse=True)
-def _thread_per_ivp_kernels(monkeypatch):
-    """These tests pin the thread-per-IVP / lane-per-dimension kernels; the cooperative small-ensemble kernel
-    that would otherwise serve their d = 1 cases has its own module (tests/test_gpu_coop.py)."""
-    monkeypatch.setenv("PN_B200_NO_COOP", "1")
-
 N_IC = 2048
 TOLS = 10.0 ** -np.arange(3, 11)
 

@@ -15,13 +15,6 @@ import problems_util as pu
 pytestmark = pytest.mark.gpu
 
 
-@pytest.fixture(autouse=True)
-def _thread_per_ivp_kernels(monkeypatch):
-    """These tests pin the thread-per-IVP / lane-per-dimension kernels; the cooperative small-ensemble kernel
-    that would otherwise serve their d = 1 cases has its own module (tests/test_gpu_coop.py)."""
-    monkeypatch.setenv("PN_B200_NO_COOP", "1")
-
-
 @pytest.fixture(scope="module")
 def cabi():
     import torch
@@ -317,7 +310,7 @@ def test_brusselator_ensemble_over_diffusion_parameter(cabi, oracle):
     assert len(set(gpu["n_accepted"][:, -1].tolist())) > 4  # members really differ
 
 
-# ---- dense factorisation with d > 1 (warp per IVP, D x D factors in shared memory) ------------------
+# ---- dense factorisation with d > 1 (register columns; D = 40: D x D factors in shared memory) -----
 DENSE_CASES = [
     ("rigid_body", 3, 2, 1, 3, pu.RIGID_BODY_PARAMS, pu.rigid_body_u0, np.linspace(0, 50, 5), dict(atol=1e-7, rtol=1e-4, dt0=50.0, corr="ts1")),
     ("rigid_body", 3, 4, 1, 3, pu.RIGID_BODY_PARAMS, pu.rigid_body_u0, np.linspace(0, 50, 5), dict(atol=1e-9, rtol=1e-6, dt0=50.0, corr="ts1")),

@@ -40,14 +40,7 @@ def _desc(_cabi, **over):
 def test_supported_and_workspace_queries_need_no_gpu(monkeypatch):
     from odecheckpts_b200 import _cabi
 
-    # the opt-in cooperative kernel for scalar ODEs has no time-sliced scheduler: header + slots only
-    n, D, K2, B2 = 5, 1, 50, 1000
-    slot = (n * n + n * D + n * (n + 1) // 2) + (n * D + n * (n + 1) // 2)
-    header2 = (256 + 2 * 128 * 4 + B2 * 8 + 255) // 256 * 256
-    monkeypatch.setenv("PN_B200_COOP_MAX_BATCH", "20000")
-    assert _cabi.workspace_bytes(_desc(_cabi, batch=B2, num_save_at=K2)) == header2 + K2 * slot * B2 * 8
     # the thread-per-IVP kernels (default)
-    monkeypatch.delenv("PN_B200_COOP_MAX_BATCH")
     d = _desc(_cabi)
     assert _cabi.supported(d)
     n, D, K, B = 5, 1, 5, 8
