@@ -2,8 +2,9 @@
 
     python code-adaptive-prob-ode-solvers_b200/build.py [--force]
 
-One translation unit per problem family, compiled in parallel; the shared library travels to the
-GPU box with the repository snapshot (it is git-ignored, not gpurun-ignored).
+One translation unit per problem family, compiled in parallel; the shared library is git-ignored.
+The kernel headers are also embedded in the library (build/pn_jit_sources.inc), for the run-time
+compilation of user-defined vector fields (csrc/pn_jit.cu); NVRTC is linked statically (README).
 """
 
 import concurrent.futures
@@ -27,6 +28,27 @@ NVCC_FLAGS = [
 ]  # fmt: skip
 
 
+# NVRTC and its device-code compiler, linked into the library (README, "User-defined vector fields")
+NVRTC_LIBS = ["-lnvrtc_static", "-lnvrtc-builtins_static", "-lnvptxcompiler_static", "-lpthread", "-ldl"]
+JIT_SOURCES = os.path.join(OBJ, "pn_jit_sources.inc")
+_DELIM = "pn_src"
+
+
+def write_jit_sources(headers):
+    """build/pn_jit_sources.inc: every csrc/*.cuh as {file name, text}; rewritten only when it changes."""
+    parts = []
+    for h in sorted(headers):
+        text = open(h, encoding="utf-8").read()
+        if f'){_DELIM}"' in text:
+            raise RuntimeError(f"{h} contains the raw-string delimiter ){_DELIM}\"")
+        parts.append(f'{{"{os.path.basename(h)}", R"{_DELIM}({text}){_DELIM}"}},\n')
+    body = "struct JitSource {\n  const char* name;\n  const char* text;\n};\nconst JitSource kJitSources[] = {\n" + "".join(parts) + "};\n"
+    old = open(JIT_SOURCES, encoding="utf-8").read() if os.path.exists(JIT_SOURCES) else None
+    if old != body:
+        with open(JIT_SOURCES, "w", encoding="utf-8") as f:
+            f.write(body)
+
+
 def _newest(paths):
     return max(os.path.getmtime(p) for p in paths)
 
@@ -39,6 +61,7 @@ def build(force=False, verbose=False):
     hdrs = glob.glob(os.path.join(CSRC, "*.cuh")) + glob.glob(os.path.join(CSRC, "*.h"))
     hdrs += [os.path.join(HERE, "..", "include", "pn_b200.h"), os.path.abspath(__file__)]
     os.makedirs(OBJ, exist_ok=True)
+    write_jit_sources(glob.glob(os.path.join(CSRC, "*.cuh")))
     dep_time = _newest(hdrs)
     jobs = []
     objs = []
@@ -51,7 +74,7 @@ def build(force=False, verbose=False):
     def compile_one(job):
         s, o = job
         extra = os.environ.get("PN_EXTRA_NVCC_FLAGS", "").split()
-        cmd = [nvcc] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + ["-c", s, "-o", o]
+        cmd = [nvcc] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + ["-I", OBJ, "-c", s, "-o", o]
         r = subprocess.run(cmd, capture_output=True, text=True)
         return s, r.returncode, r.stdout + r.stderr
 
@@ -63,7 +86,7 @@ def build(force=False, verbose=False):
                 if rc:
                     raise RuntimeError(f"nvcc failed on {s}")
     if jobs or not os.path.exists(LIB) or os.path.getmtime(LIB) < _newest(objs):
-        cmd = [nvcc, "-shared", "-o", LIB] + objs + ["-gencode", "arch=compute_100a,code=sm_100a"]
+        cmd = [nvcc, "-shared", "-o", LIB] + objs + ["-gencode", "arch=compute_100a,code=sm_100a"] + NVRTC_LIBS
         r = subprocess.run(cmd, capture_output=True, text=True)
         if r.returncode:
             sys.stderr.write(r.stdout + r.stderr)

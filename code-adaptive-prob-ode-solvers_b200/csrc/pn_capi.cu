@@ -14,6 +14,7 @@
 #include <vector>
 
 #include "../../include/pn_b200.h"
+#include "pn_jit.h"
 #include "pn_registry.h"
 
 namespace pn {
@@ -24,13 +25,14 @@ static std::vector<KernelEntry>& table() {
 }
 void register_kernel(const KernelEntry& e) { table().push_back(e); }
 const KernelEntry* find_kernel(int family, int problem, int nu, int strategy, int d) {
+  if (jit_is_user_problem(problem)) return jit_find(family, problem, nu, strategy, d);
   for (const auto& e : table())
     if (e.family == family && e.problem == problem && e.nu == nu && e.strategy == strategy && e.D == d) return &e;
   return nullptr;
 }
 
 static thread_local std::string g_err;
-static int fail(int code, const std::string& msg) {
+int fail(int code, const std::string& msg) {
   g_err = msg;
   return code;
 }
@@ -322,6 +324,10 @@ static int make_plan(const pn_b200_desc* d, Plan* p, bool need_device) {
     }
   }
   if (!need_device) return PN_B200_SUCCESS;
+  if (p->k->jit) {
+    rc = jit_load(p->k);
+    if (rc) return rc;
+  }
   int dev = 0;
   cudaError_t ce = cudaGetDevice(&dev);
   if (ce != cudaSuccess) return fail(PN_B200_ERR_CUDA, cudaGetErrorString(ce));
@@ -422,6 +428,13 @@ size_t pn_b200_workspace_bytes(const pn_b200_desc* desc) {
   Plan p;
   if (make_plan(desc, &p, false)) return 0;
   return p.ws_ticket + p.ws_cond + p.ws_wide + p.ws_slice + p.ws_mle;
+}
+
+int pn_b200_compile(const pn_b200_desc* desc) {
+  const KernelEntry* k = nullptr;
+  int rc = resolve(desc, &k);
+  if (rc == PN_B200_SUCCESS && k->jit) rc = jit_load(k);
+  return rc;
 }
 
 int pn_b200_output_sizes(const pn_b200_desc* desc, pn_b200_sizes* sz) {
@@ -544,7 +557,7 @@ int pn_b200_solve_save_at(const pn_b200_desc* desc, const double* u0, const doub
   // time-sliced scheduling: uniform tolerances only (ragged ensembles get the longest-first order
   // above instead), and only when the ensemble does not fit the resident lanes anyway
   bool sliced = false;
-  if (p.ws_slice > 0 && p.k->launch_solve_sliced && !tol && desc->batch > (int64_t)p.grid * p.k->threads &&
+  if (p.ws_slice > 0 && p.k->solve_func_sliced && !tol && desc->batch > (int64_t)p.grid * p.k->threads &&
       !getenv("PN_B200_NO_SLICE")) {
     char* base = (char*)workspace + p.ws_ticket + p.ws_cond + p.ws_wide;
     ce = cudaMemsetAsync(base, 0xff, p.ws_queue, stream);
@@ -574,7 +587,10 @@ int pn_b200_solve_save_at(const pn_b200_desc* desc, const double* u0, const doub
     }
   }
   if (prof) cudaEventRecord(g_ev[0], stream);
-  ce = sliced ? p.k->launch_solve_sliced(a, p.grid, p.smem, stream) : p.k->launch_solve(a, p.grid, p.smem, stream);
+  if (p.k->jit)
+    ce = jit_launch_solve(p.k, sliced, a, p.grid, p.smem, stream);
+  else
+    ce = sliced ? p.k->launch_solve_sliced(a, p.grid, p.smem, stream) : p.k->launch_solve(a, p.grid, p.smem, stream);
   if (ce != cudaSuccess) return fail(PN_B200_ERR_CUDA, std::string("solve kernel launch: ") + cudaGetErrorString(ce));
   if (prof) {
     cudaEventRecord(g_ev[1], stream);
@@ -596,7 +612,7 @@ int pn_b200_solve_save_at(const pn_b200_desc* desc, const double* u0, const doub
   s.u_std = u_std;
   s.marg_mean = marg_mean;
   s.marg_chol = marg_chol;
-  ce = p.k->launch_smooth(s, stream);
+  ce = p.k->jit ? jit_launch_smooth(p.k, s, stream) : p.k->launch_smooth(s, stream);
   if (ce != cudaSuccess) return fail(PN_B200_ERR_CUDA, std::string("smoothing kernel launch: ") + cudaGetErrorString(ce));
   if (prof) {
     cudaEventRecord(g_ev[3], stream);
@@ -610,8 +626,9 @@ int pn_b200_markov_sample(const pn_b200_desc* desc, const void* workspace, size_
                           void* cuda_stream) {
   Plan p;
   int rc = make_plan(desc, &p, false);
+  if (rc == PN_B200_SUCCESS && p.k->jit) rc = jit_load(p.k);
   if (rc) return rc;
-  if (desc->strategy != PN_B200_FIXEDPOINT || !p.k->launch_sample)
+  if (desc->strategy != PN_B200_FIXEDPOINT || !(p.k->launch_sample || p.k->sample_func))
     return fail(PN_B200_ERR_UNSUPPORTED, "posterior sampling needs a fixed-point solve");
   if (!workspace || workspace_bytes < p.ws_ticket + p.ws_cond || !samples || !status || num_samples < 1)
     return fail(PN_B200_ERR_ARGUMENT, "bad sampling arguments");
@@ -626,7 +643,7 @@ int pn_b200_markov_sample(const pn_b200_desc* desc, const void* workspace, size_
   a.cond = (const double*)((const char*)workspace + p.ws_ticket);
   a.status = status;
   a.samples = samples;
-  cudaError_t ce = p.k->launch_sample(a, (cudaStream_t)cuda_stream);
+  cudaError_t ce = p.k->jit ? jit_launch_sample(p.k, a, (cudaStream_t)cuda_stream) : p.k->launch_sample(a, (cudaStream_t)cuda_stream);
   if (ce != cudaSuccess) return fail(PN_B200_ERR_CUDA, std::string("sampling kernel launch: ") + cudaGetErrorString(ce));
   return PN_B200_SUCCESS;
 }
@@ -636,8 +653,9 @@ int pn_b200_log_marginal_likelihood(const pn_b200_desc* desc, const void* worksp
                                     double* lml, void* cuda_stream) {
   Plan p;
   int rc = make_plan(desc, &p, false);
+  if (rc == PN_B200_SUCCESS && p.k->jit) rc = jit_load(p.k);
   if (rc) return rc;
-  if (desc->strategy != PN_B200_FIXEDPOINT || !p.k->launch_lml)
+  if (desc->strategy != PN_B200_FIXEDPOINT || !(p.k->launch_lml || p.k->lml_func))
     return fail(PN_B200_ERR_UNSUPPORTED, "the log marginal likelihood needs a fixed-point solve of the thread-per-IVP, lane-per-dimension or CTA-per-IVP isotropic family");
   if (!workspace || workspace_bytes < p.ws_ticket + p.ws_cond || !status || !data || !obs_std || !lml)
     return fail(PN_B200_ERR_ARGUMENT, "bad likelihood arguments");
@@ -663,7 +681,7 @@ int pn_b200_log_marginal_likelihood(const pn_b200_desc* desc, const void* worksp
   if (ce != cudaSuccess) return fail(PN_B200_ERR_CUDA, std::string("cudaMallocAsync: ") + cudaGetErrorString(ce));
   a.w = scratch;
   a.logs = scratch + nw;
-  ce = p.k->launch_lml(a, stream);
+  ce = p.k->jit ? jit_launch_lml(p.k, a, stream) : p.k->launch_lml(a, stream);
   cudaFreeAsync(scratch, stream);
   if (ce != cudaSuccess) return fail(PN_B200_ERR_CUDA, std::string("likelihood kernel launch: ") + cudaGetErrorString(ce));
   return PN_B200_SUCCESS;

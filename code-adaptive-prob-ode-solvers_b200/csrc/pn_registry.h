@@ -44,6 +44,12 @@ struct KernelEntry {
   cudaError_t (*launch_smooth)(const SmoothArgs&, cudaStream_t);
   cudaError_t (*launch_sample)(const SampleArgs&, cudaStream_t) = nullptr;  // nullptr: family has no sampler yet
   cudaError_t (*launch_lml)(const LmlArgs&, cudaStream_t) = nullptr;        // nullptr: no likelihood kernel for this family
+  // run-time compiled builds of user problems (pn_jit.cu): the launch_* pointers stay null; the kernels are library
+  // handles, set once jit_load has compiled the module, and are launched with cudaLaunchKernel (jit_launch_*)
+  bool jit = false;
+  const void* smooth_func = nullptr;
+  const void* sample_func = nullptr;  // nullptr: no sampler
+  const void* lml_func = nullptr;     // likelihood sweep; nullptr: no likelihood kernel
 };
 
 void register_kernel(const KernelEntry& e);

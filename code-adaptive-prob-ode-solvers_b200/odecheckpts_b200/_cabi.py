@@ -21,6 +21,8 @@ PROBLEM_IDS = {
     "van_der_pol": 5,
     "lotka_volterra": 6,
 }
+USER_PROBLEM_BASE = 1024  # ids of problems registered at run time (register_problem) start here
+SOURCE_FORMS = {"simple": 0, "full": 1}
 FACTORISATIONS = {"isotropic": 0, "blockdiag": 1, "dense": 2}
 CORRECTIONS = {"ts0": 0, "ts1": 1}
 STRATEGIES = {"filter": 0, "fixedpoint": 1}
@@ -96,6 +98,9 @@ EXPORTS = (
     "pn_b200_set_profiling",
     "pn_b200_get_last_timing",
     "pn_b200_last_error",
+    "pn_b200_register_problem",
+    "pn_b200_problem_evaluate",
+    "pn_b200_compile",
 )
 
 _lib = None
@@ -142,6 +147,13 @@ def lib():
         L.pn_b200_get_last_timing.argtypes = [C.POINTER(C.c_float), C.POINTER(C.c_float)]
         L.pn_b200_last_error.restype = C.c_char_p
         L.pn_b200_last_error.argtypes = []
+        L.pn_b200_register_problem.restype = C.c_int
+        L.pn_b200_register_problem.argtypes = [C.c_char_p, C.c_char_p, C.c_int, C.c_int32, C.c_int32, C.c_int32,
+                                               C.POINTER(C.c_int32)]  # fmt: skip
+        L.pn_b200_problem_evaluate.restype = C.c_int
+        L.pn_b200_problem_evaluate.argtypes = [C.c_int32, C.c_int32, C.c_int64] + [vp] * 6
+        L.pn_b200_compile.restype = C.c_int
+        L.pn_b200_compile.argtypes = [C.POINTER(Desc)]
         _lib = L
     return _lib
 
@@ -174,6 +186,51 @@ def output_sizes(desc):
     sz = Sizes()
     check(lib().pn_b200_output_sizes(C.byref(desc), C.byref(sz)))
     return {name: int(getattr(sz, name)) for name, _ in Sizes._fields_}
+
+
+def register_problem(name, source, *, d, ode_order=1, num_params=0, form="simple"):
+    """Compile a user-defined vector field (CUDA C++ source, see include/pn_b200.h) and return its problem id.
+    A compile error raises ValueError with the compiler log."""
+    if form not in SOURCE_FORMS:
+        raise ValueError(f"form must be one of {sorted(SOURCE_FORMS)}")
+    pid = C.c_int32(-1)
+    check(lib().pn_b200_register_problem(name.encode(), source.encode(), SOURCE_FORMS[form], int(d), int(ode_order),
+                                         int(num_params), C.byref(pid)))  # fmt: skip
+    return pid.value
+
+
+def compile_kernels(desc):
+    """Compile and load the kernels that serve `desc` now (user problems; a no-op for built-in ones)."""
+    check(lib().pn_b200_compile(C.byref(desc)))
+
+
+def problem_evaluate_device(problem, nu, u0, params, *, d, ode_order, f=True, taylor=True, jac=True, stream=None):
+    """The functor of `problem` at n states u0 [n, ode_order, d] (torch CUDA float64): dict with f [n, d],
+    taylor [n, nu + 1, d] (the Taylor-mode initialisation) and jac [n, d, ode_order * d], as requested."""
+    import torch
+
+    dev = u0.device
+    n = u0.shape[0]
+    u0 = u0.to(torch.float64).contiguous()
+    params = None if params is None else params.to(device=dev, dtype=torch.float64).contiguous()
+    f64 = dict(dtype=torch.float64, device=dev)
+    out = {}
+    if f:
+        out["f"] = torch.empty((n, d), **f64)
+    if taylor:
+        out["taylor"] = torch.empty((n, nu + 1, d), **f64)
+    if jac:
+        out["jac"] = torch.empty((n, d, ode_order * d), **f64)
+
+    def ptr(x):
+        return None if x is None else C.c_void_p(x.data_ptr())
+
+    s = torch.cuda.current_stream(dev) if stream is None else stream
+    with torch.cuda.device(dev):
+        rc = lib().pn_b200_problem_evaluate(int(problem), int(nu), int(n), ptr(u0), ptr(params), ptr(out.get("f")),
+                                            ptr(out.get("taylor")), ptr(out.get("jac")), C.c_void_p(s.cuda_stream))  # fmt: skip
+    check(rc)
+    return out
 
 
 def kernel_info(desc):

@@ -7,12 +7,16 @@ convention ``vf(*u, t=..., p=...)`` (src/odecheckpts/ivpsolvers.py:59-60) so use
 it in lambdas keeps working: the solver discovers the functor behind any wrapper by calling
 it once with tracer arguments (the moral equivalent of jax tracing).  Called with real
 arrays it evaluates the same formula with numpy on the host (handy for truth solutions).
+
+Other ODEs: :func:`cuda_vector_field` compiles a user's CUDA C++ vector field at run time into
+the same kernels.
 """
 
 import threading
 
 import numpy as np
 
+from . import _cabi
 from ._cabi import PROBLEM_IDS
 
 _trace = threading.local()
@@ -26,9 +30,9 @@ class _Tracer:
 
 
 class VectorField:
-    def __init__(self, name, d, ode_order, num_params, fun):
+    def __init__(self, name, d, ode_order, num_params, fun, problem_id=None):
         self.name = name
-        self.problem_id = PROBLEM_IDS[name]
+        self.problem_id = PROBLEM_IDS[name] if problem_id is None else problem_id
         self.d = d
         self.ode_order = ode_order
         self.num_params = num_params
@@ -40,6 +44,8 @@ class VectorField:
             if rec is not None:
                 rec.append((self, p))
             return _Tracer(u[0].shape)
+        if self._fun is None:
+            raise TypeError(f"{self.name}: no host function was given (cuda_vector_field(..., host=...))")
         return self._fun(*[np.asarray(x, dtype=np.float64) for x in u], *_flat_params(p))
 
     def __repr__(self):
@@ -72,9 +78,29 @@ def resolve_vector_field(vf, u0, t0=0.0):
         raise TypeError(
             "the vector field must be (a wrapper around) one odecheckpts_b200.ivps VectorField: vector "
             "fields are compiled into the CUDA kernels as device functors, arbitrary Python callables "
-            "cannot run on the GPU"
+            "cannot run on the GPU; write the vector field in CUDA C++ with ivps.cuda_vector_field"
         )
     return records[0]
+
+
+def cuda_vector_field(name, source, *, d, ode_order=1, num_params=0, form="simple", host=None):
+    """A user-defined vector field, compiled at run time into the solver kernels.
+
+    ``source`` is CUDA C++.  ``form="simple"``: one function templated on the number type,
+
+        template <class T> PN_DEV void vf(const T* u, const double* p, T* f)
+
+    with u = (u, u', ...) of length ode_order * d, p the num_params parameters and f of length d;
+    T is double or a truncated Taylor series (pn::Jet), so use arithmetic, fma, sqrt, rcp, exp, log,
+    sin, cos and pow.  An optional ``PN_DEV void jac(const double* u, const double* p, double* J)``
+    (J[d][ode_order * d]) replaces the derived Jacobian.  ``form="full"``: a ``struct Problem`` with the
+    interface of the built-in functors (csrc/pn_problems.cuh).  Compile errors raise ValueError with
+    the compiler log; its line numbers are the lines of ``source``.
+
+    ``host`` is an optional numpy function ``host(*u, *params)`` kept for truth solutions; it is
+    what the returned VectorField evaluates when called with arrays."""
+    pid = _cabi.register_problem(name, source, d=d, ode_order=ode_order, num_params=num_params, form=form)
+    return VectorField(name, d, ode_order, num_params, host, problem_id=pid)
 
 
 # ---- the zoo ---------------------------------------------------------------------------------

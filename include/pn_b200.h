@@ -184,6 +184,51 @@ int pn_b200_measure_fp64_peak(double* tflops, void* cuda_stream);
 int pn_b200_set_profiling(int enable);
 int pn_b200_get_last_timing(float* solve_ms, float* smooth_ms);
 
+/*
+ * User-defined vector fields, compiled at run time (NVRTC) into the same kernels the built-in problems use.
+ *
+ * `source` is CUDA C++ in one of two forms:
+ *   PN_B200_FORM_SIMPLE  template <class T> PN_DEV void vf(const T* u, const double* p, T* f)
+ *                        u = (u, u', ...)[ode_order * d], p[num_params], f[d]; T is double or pn::Jet<N> (truncated
+ *                        Taylor series).  Optionally  PN_DEV void jac(const double* u, const double* p, double* J)
+ *                        with J[d][ode_order * d]; without it the Jacobian is derived from vf on pn::Jet<2>.
+ *   PN_B200_FORM_FULL    struct Problem with the interface of the built-in functors (csrc/pn_problems.cuh):
+ *                        D, Q, P, HAS_JAC, vf, jac, vf_jet<N>.
+ * Registration compiles a check kernel: a compile error returns PN_B200_ERR_ARGUMENT, and pn_b200_last_error()
+ * holds the whole compiler log, whose line numbers are the lines of `source` under the file name `name`
+ * ([A-Za-z0-9_.-], at most 128 characters).  Registering the same (name, source, form, sizes) again returns the
+ * same id.  d in 1 .. 32, ode_order 1 or 2, num_params 0 .. 64.  The source lives in a namespace of its own in
+ * which the names Prob, PnSource, PN_HAS_JAC and pn_no_jac are taken.  Ids are handed out in registration order,
+ * so processes that register the same problems in the same order (the ranks of a multi-GPU run) share ids.
+ *
+ * A user problem id (>= PN_B200_USER_PROBLEM_BASE) goes into pn_b200_desc.problem like a built-in one.  Its kernels
+ * are compiled on first use per (kernel family, nu, strategy) and cached for the life of the process: the first
+ * solve, pn_b200_get_kernel_info or pn_b200_compile of a configuration compiles, pn_b200_supported and
+ * pn_b200_workspace_bytes never do.  Builds: the thread-per-IVP kernels (d <= 3; the small-ensemble build for the
+ * fixed-point strategy with d <= 2), the lane-per-dimension kernels (isotropic and blockdiag, d <= 32) and the
+ * dense register-column kernel ((nu + 1) d <= 32).
+ */
+enum { PN_B200_USER_PROBLEM_BASE = 1024 };
+enum { PN_B200_FORM_SIMPLE = 0, PN_B200_FORM_FULL = 1 };
+int pn_b200_register_problem(const char* name, const char* source, int form, int32_t d, int32_t ode_order,
+                             int32_t num_params, int32_t* problem_id);
+
+/* Compiles (and loads) the kernels that serve `desc` now, so that a later timed solve does not include the
+ * compilation.  A no-op for built-in problems. */
+int pn_b200_compile(const pn_b200_desc* desc);
+
+/*
+ * Evaluates a problem's functor for n states (DEVICE pointers, stream-ordered): u0 [n][ode_order][d],
+ * params [n][P] (P: the problem's parameter count); outputs, each optional (NULL: not computed):
+ *   f      [n][d]              the vector field at u0
+ *   taylor [n][nu + 1][d]      the Taylor coefficients u^(k)(t0), k = 0 .. nu, the solver's initialisation
+ *   jac    [n][d][ode_order d] the Jacobian (PN_B200_ERR_UNSUPPORTED for a problem without one)
+ * For user problems and for the built-in problems of fixed size (all but the Brusselator), whose functors are
+ * compiled for this the same way.
+ */
+int pn_b200_problem_evaluate(int32_t problem, int32_t nu, int64_t n, const double* u0, const double* params, double* f,
+                             double* taylor, double* jac, void* cuda_stream);
+
 /* Human-readable description of the last error on the calling thread. */
 const char* pn_b200_last_error(void);
 
