@@ -206,7 +206,7 @@ __global__ void __launch_bounds__(32 * WARPS) pn_dense_kernel(const __grid_const
       double u0[Q * d], tc[N][d];
 #pragma unroll
       for (int i = 0; i < Q * d; ++i) u0[i] = a.u0[b * (Q * d) + i];
-      taylor_init<Prob, NU>(u0, par, tc);
+      taylor_init<Prob, NU>(u0, a.save_at[0], par, tc);
       if (lane == 0) {
 #pragma unroll
         for (int i = 0; i < N; ++i)

@@ -224,7 +224,7 @@ __global__ void __launch_bounds__(32 * WARPS) pn_dense_rows_kernel(const __grid_
           double u0[Q * d], tc[N][d];
 #pragma unroll
           for (int i = 0; i < Q * d; ++i) u0[i] = a.u0[b * (Q * d) + i];
-          taylor_init<Prob, NU>(u0, par, tc);
+          taylor_init<Prob, NU>(u0, a.save_at[0], par, tc);
           if (c == 0) {
 #pragma unroll
             for (int i = 0; i < N; ++i)
@@ -308,13 +308,21 @@ __global__ void __launch_bounds__(32 * WARPS) pn_dense_rows_kernel(const __grid_
       }
     }
     __syncwarp();
-    // linearise: every lane evaluates the (tiny) vector field redundantly in registers
+    // linearise: every lane evaluates the (tiny) vector field redundantly in registers; a time-dependent problem at
+    // the time the prediction reaches (the same double an accepted step or a checkpoint commits as the new time)
     double zv[d];
     {
+      double t_vf = 0.0;
+      if constexpr (TimeDependent<Prob>::value) {
+        if (mode == MODE_STEP)
+          t_vf = (a.flags & FLAG_FIXED_GRID) ? t_ck : (t + dt);
+        else
+          t_vf = (mode == MODE_INTERP_A) ? t_ck : pend_t;
+      }
       double uarg[Q * d], f[d];
 #pragma unroll
       for (int k = 0; k < Q * d; ++k) uarg[k] = m_ext[k];
-      Prob::vf(uarg, par, f);
+      vf_at<Prob>(uarg, t_vf, par, f);
 #pragma unroll
       for (int l = 0; l < d; ++l) zv[l] = m_ext[Q * d + l] - f[l];
       for (int e = c; e < d * Dn; e += LANES) H[e] = 0.0;
@@ -325,7 +333,7 @@ __global__ void __launch_bounds__(32 * WARPS) pn_dense_rows_kernel(const __grid_
       }
       if (Prob::HAS_JAC && a.correction == 1) {
         double J[d * Q * d];
-        Prob::jac(uarg, par, J);
+        jac_at<Prob>(uarg, t_vf, par, J);
         if (c == 0) {
 #pragma unroll
           for (int l = 0; l < d; ++l)

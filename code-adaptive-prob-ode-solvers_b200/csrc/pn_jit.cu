@@ -131,27 +131,39 @@ bool valid_name(const std::string& s) {
   return true;
 }
 
-// The user's text in its own namespace, then the Prob functor the kernels are instantiated with.
+// The user's text in its own namespace, then the Prob functor the kernels are instantiated with.  A time-dependent
+// problem's functions take the time after the state (pn_user_problem.cuh).
 std::string problem_text(const ProblemRec& r) {
   const std::string ns = "pn_user_" + std::to_string(r.id);
+  const bool time = (r.form & PN_B200_FORM_TIME_DEPENDENT) != 0;
+  const int form = r.form & ~PN_B200_FORM_TIME_DEPENDENT;
   std::string s = "namespace " + ns + " {\nusing namespace ::pn::jet;\n";
-  if (r.form == PN_B200_FORM_SIMPLE) {
+  if (form == PN_B200_FORM_SIMPLE) {
     // a Jacobian the user does not define resolves to this declaration (never defined: only its type is used)
     s += "struct pn_no_jac {};\ntemplate <class... A> pn_no_jac jac(A...);\n";
   }
   s += "#line 1 \"" + r.name + "\"\n" + r.source + "\n#line 1 \"" + r.name + " (adapter)\"\n}\nnamespace " + ns + " {\n";
   const std::string dims = std::to_string(r.d) + ", " + std::to_string(r.q) + ", " + std::to_string(r.P);
-  if (r.form == PN_B200_FORM_SIMPLE) {
+  if (form == PN_B200_FORM_SIMPLE && !time) {
     s += "struct PnSource {\n"
          "  template <class T> PN_DEV static void vf(const T* u, const double* p, T* f) { ::" + ns + "::vf<T>(u, p, f); }\n"
          "  template <int Z = 0> PN_DEV static void jac(const double* u, const double* p, double* J) { ::" + ns + "::jac(u, p, J); }\n"
          "};\n"
          "constexpr bool PN_HAS_JAC = !::pn::jet::IsSame<decltype(::" + ns + "::jac((const double*)0, (const double*)0, (double*)0)), pn_no_jac>::value;\n"
          "using Prob = ::pn::UserProblem<PnSource, " + dims + ", PN_HAS_JAC>;\n";
+  } else if (form == PN_B200_FORM_SIMPLE) {
+    s += "struct PnSource {\n"
+         "  template <class T> PN_DEV static void vf(const T* u, const T& t, const double* p, T* f) { ::" + ns + "::vf<T>(u, t, p, f); }\n"
+         "  template <int Z = 0> PN_DEV static void jac(const double* u, double t, const double* p, double* J) { ::" + ns + "::jac(u, t, p, J); }\n"
+         "};\n"
+         "constexpr bool PN_HAS_JAC = !::pn::jet::IsSame<decltype(::" + ns + "::jac((const double*)0, 0.0, (const double*)0, (double*)0)), pn_no_jac>::value;\n"
+         "using Prob = ::pn::UserProblem<PnSource, " + dims + ", PN_HAS_JAC, true>;\n";
   } else {
     s += "static_assert(Problem::D == " + std::to_string(r.d) + ", \"Problem::D differs from the registered d\");\n"
          "static_assert(Problem::Q == " + std::to_string(r.q) + ", \"Problem::Q differs from the registered ode_order\");\n"
          "static_assert(Problem::P == " + std::to_string(r.P) + ", \"Problem::P differs from the registered num_params\");\n"
+         "static_assert(::pn::TimeDependent<Problem>::value == " + (time ? "true" : "false") +
+         ", \"Problem::TIME differs from the registered time dependence\");\n"
          "using Prob = ::pn::FullProblem<Problem>;\n";
   }
   s += "}\n";
@@ -421,7 +433,8 @@ int pn_b200_register_problem(const char* name, const char* source, int form, int
                              int32_t num_params, int32_t* problem_id) {
   if (!name || !source || !problem_id) return fail(PN_B200_ERR_ARGUMENT, "null name, source or problem_id");
   if (!valid_name(name)) return fail(PN_B200_ERR_ARGUMENT, "problem name: 1 to 128 characters of [A-Za-z0-9_.-]");
-  if (form != PN_B200_FORM_SIMPLE && form != PN_B200_FORM_FULL) return fail(PN_B200_ERR_ARGUMENT, "unknown source form");
+  const int base_form = form & ~PN_B200_FORM_TIME_DEPENDENT;
+  if (base_form != PN_B200_FORM_SIMPLE && base_form != PN_B200_FORM_FULL) return fail(PN_B200_ERR_ARGUMENT, "unknown source form");
   if (d < 1 || d > MAX_DIM) return fail(PN_B200_ERR_ARGUMENT, "d must be in 1 .. 32");
   if (ode_order != 1 && ode_order != 2) return fail(PN_B200_ERR_ARGUMENT, "ode_order must be 1 or 2");
   if (num_params < 0 || num_params > MAX_PARAMS) return fail(PN_B200_ERR_ARGUMENT, "num_params must be in 0 .. 64");
@@ -447,6 +460,11 @@ int pn_b200_register_problem(const char* name, const char* source, int form, int
 
 int pn_b200_problem_evaluate(int32_t problem, int32_t nu, int64_t n, const double* u0, const double* params, double* f,
                              double* taylor, double* jac, void* cuda_stream) {
+  return pn_b200_problem_evaluate_at(problem, nu, n, nullptr, u0, params, f, taylor, jac, cuda_stream);
+}
+
+int pn_b200_problem_evaluate_at(int32_t problem, int32_t nu, int64_t n, const double* t, const double* u0, const double* params,
+                                double* f, double* taylor, double* jac, void* cuda_stream) {
   if (nu < 1 || nu > 8) return fail(PN_B200_ERR_ARGUMENT, "nu must be in 1 .. 8");
   if (n < 0) return fail(PN_B200_ERR_ARGUMENT, "n must be >= 0");
   int P = 0;
@@ -474,7 +492,7 @@ int pn_b200_problem_evaluate(int32_t problem, int32_t nu, int64_t n, const doubl
   if (!u0 || (P > 0 && !params)) return fail(PN_B200_ERR_ARGUMENT, "null u0 or params");
   long long nn = n;
   int np = P;
-  void* args[] = {&nn, &np, &u0, &params, &f, &taylor, &jac};
+  void* args[] = {&nn, &np, &t, &u0, &params, &f, &taylor, &jac};
   cudaError_t ce = cudaLaunchKernel(m->kernels[0], dim3((unsigned)((n + 127) / 128)), dim3(128), args, 0, (cudaStream_t)cuda_stream);
   if (ce != cudaSuccess) return fail(PN_B200_ERR_CUDA, std::string("evaluation kernel launch: ") + cudaGetErrorString(ce));
   return PN_B200_SUCCESS;

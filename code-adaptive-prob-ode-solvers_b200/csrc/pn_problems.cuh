@@ -9,6 +9,10 @@
 //   jac(u, par, J)    J[D][Q*D]  (HAS_JAC)
 //   vf_jet<N>(U, par, F)  the same expression on truncated power series (normalised Taylor
 //                     coefficients), used once per member for the initial state.
+//   TIME              optional, false when absent: the problem is time-dependent and its functions take
+//                     the time after the state: vf(u, t, par, f), jac(u, t, par, J) and vf_jet<N>(U, Tc, par, F)
+//                     with Tc[N] the time's normalised Taylor coefficients.  The kernels call the three through
+//                     vf_at / jac_at / taylor_init, which pass the time to a time-dependent problem only.
 // Fixed-size problems only; the Brusselator (d = 2N) lives in the CTA-per-IVP kernel.
 #pragma once
 #include "pn_math.cuh"
@@ -346,9 +350,35 @@ struct BrusselatorWide {
   }
 };
 
-// taylor.odejet_padded_scan replacement: tc[k][l] = u_l^{(k)}(t0), k = 0..NU.
+// ---- time-dependent problems (TIME) ------------------------------------------------------
+template <class Prob, class = void>
+struct TimeDependent {
+  static constexpr bool value = false;
+};
+template <class Prob>
+struct TimeDependent<Prob, decltype(void(Prob::TIME))> {
+  static constexpr bool value = Prob::TIME;
+};
+template <class Prob>
+PN_DEV void vf_at(const double* u, double t, const double* par, double* f) {
+  if constexpr (TimeDependent<Prob>::value)
+    Prob::vf(u, t, par, f);
+  else
+    Prob::vf(u, par, f);
+}
+template <class Prob>
+PN_DEV void jac_at(const double* u, double t, const double* par, double* J) {
+  if constexpr (TimeDependent<Prob>::value)
+    Prob::jac(u, t, par, J);
+  else
+    Prob::jac(u, par, J);
+}
+
+// taylor.odejet_padded_scan replacement: tc[k][l] = u_l^{(k)}(t0), k = 0..NU.  A time-dependent field sees the
+// time as the series t0 + (t - t0), coefficients (t0, 1, 0, ...): the recursion then yields the exact derivatives
+// of a non-autonomous ODE, where a time frozen at t0 would leave all but the first derivative wrong.
 template <class Prob, int NU>
-PN_DEV void taylor_init(const double* u0 /*[Q*D]*/, const double* par, double (&tc)[NU + 1][Prob::D]) {
+PN_DEV void taylor_init(const double* u0 /*[Q*D]*/, double t0, const double* par, double (&tc)[NU + 1][Prob::D]) {
   constexpr int N = NU + 1, D = Prob::D, Q = Prob::Q;
   double C[D * N], U[Q * D * N], F[D * N];
 #pragma unroll
@@ -369,7 +399,14 @@ PN_DEV void taylor_init(const double* u0 /*[Q*D]*/, const double* par, double (&
         for (int i = 0; i < N; ++i) U[(D + l) * N + i] = (i + 1 < N) ? (double)(i + 1) * C[l * N + i + 1] : 0.0;
       }
     }
-    Prob::template vf_jet<N>(U, par, F);
+    if constexpr (TimeDependent<Prob>::value) {
+      double Tc[N];
+#pragma unroll
+      for (int i = 0; i < N; ++i) Tc[i] = (i == 0) ? t0 : ((i == 1) ? 1.0 : 0.0);
+      Prob::template vf_jet<N>(U, Tc, par, F);
+    } else {
+      Prob::template vf_jet<N>(U, par, F);
+    }
 #pragma unroll
     for (int l = 0; l < D; ++l) {
       if (Q == 1)

@@ -307,17 +307,18 @@ PN_DEV double group_sum(double v, unsigned gmask) {
 
 // Vector field for the lane-per-dimension kernels: every lane holds ITS dimension's predicted
 // (u, u', ...) and gets back ITS component of f.  Default: gather everything with shuffles,
-// evaluate the whole field, select the own component.
+// evaluate the whole field, select the own component.  t: the time of the evaluation (read by
+// time-dependent problems only).
 template <class Prob, int GROUP>
 struct GroupVf {
-  PN_DEV static double eval(const double* own /*[Q]*/, int sub, int base, unsigned gmask, const double* par) {
+  PN_DEV static double eval(const double* own /*[Q]*/, int sub, int base, unsigned gmask, double t, const double* par) {
     constexpr int DT = Prob::D, Q = Prob::Q;
     double u[Q * DT], f[DT];
 #pragma unroll
     for (int k = 0; k < Q; ++k)
 #pragma unroll
       for (int c = 0; c < DT; ++c) u[k * DT + c] = __shfl_sync(gmask, own[k], base + c);
-    Prob::vf(u, par, f);
+    vf_at<Prob>(u, t, par, f);
     double r = f[0];
 #pragma unroll
     for (int c = 1; c < DT; ++c) r = (sub == c) ? f[c] : r;
@@ -328,7 +329,7 @@ struct GroupVf {
 // Pleiades: lane c < 7 owns x_c, lane 7 + i owns y_i; each lane sums its 6 pair terms.
 template <int GROUP>
 struct GroupVf<Pleiades, GROUP> {
-  PN_DEV static double eval(const double* own, int sub, int base, unsigned gmask, const double*) {
+  PN_DEV static double eval(const double* own, int sub, int base, unsigned gmask, double, const double*) {
     const int i = (sub < 7) ? sub : ((sub < 14) ? sub - 7 : 0);
     const bool isx = sub < 7;
     const double xi = __shfl_sync(gmask, own[0], base + i);
@@ -350,7 +351,7 @@ struct GroupVf<Pleiades, GROUP> {
 // Brusselator: lane i < N owns u_i, lane N + i owns v_i; nearest-neighbour stencil by shuffles.
 template <int NPTS, int GROUP>
 struct GroupVf<Brusselator<NPTS>, GROUP> {
-  PN_DEV static double eval(const double* own, int sub, int base, unsigned gmask, const double* par) {
+  PN_DEV static double eval(const double* own, int sub, int base, unsigned gmask, double, const double* par) {
     const bool isu = sub < NPTS;
     const int i = isu ? sub : sub - NPTS;
     const double c = par[0] * (double)((NPTS + 1) * (NPTS + 1));
@@ -1139,7 +1140,7 @@ __global__ void __launch_bounds__(THREADS * (1 + PAIR) + 64 * PIPE, (PIPE || PAI
           for (int i = 0; i < N; ++i) SM(i, 0) = 0.0;  // dummy register column
         } else {
           double tc[N][DT];
-          taylor_init<Prob, NU>(u0, par, tc);
+          taylor_init<Prob, NU>(u0, a.save_at[0], par, tc);
 #pragma unroll
           for (int i = 0; i < N; ++i) {
             if constexpr (GROUP == 1) {
@@ -1333,13 +1334,21 @@ __global__ void __launch_bounds__(THREADS * (1 + PAIR) + 64 * PIPE, (PIPE || PAI
         m_ext_p[i][c] = acc;
         m_ext[i][c] = p[i] * acc;
       }
-    // linearise at the predicted mean
+    // linearise at the predicted mean, at the time this iteration's prediction reaches (for a time-dependent
+    // problem; the same double an accepted step or a checkpoint commits as the new time)
+    double t_vf = 0.0;
+    if constexpr (TimeDependent<Prob>::value) {
+      if (mode == MODE_STEP)
+        t_vf = (a.flags & FLAG_FIXED_GRID) ? t_ck : (t + dt);
+      else
+        t_vf = (mode == MODE_INTERP_A) ? t_ck : SPEND(0);
+    }
     double z[D], h[Q + 1];
     if (GROUP > 1) {
       double own[Q];
 #pragma unroll
       for (int k = 0; k < Q; ++k) own[k] = m_ext[k][0];
-      const double f_own = GroupVf<Prob, GROUP>::eval(own, sub, base, gmask, par);
+      const double f_own = GroupVf<Prob, GROUP>::eval(own, sub, base, gmask, t_vf, par);
       z[0] = m_ext[Q][0] - f_own;
 #pragma unroll
       for (int k = 0; k < Q; ++k) h[k] = 0.0;
@@ -1350,7 +1359,7 @@ __global__ void __launch_bounds__(THREADS * (1 + PAIR) + 64 * PIPE, (PIPE || PAI
       for (int k = 0; k < Q; ++k)
 #pragma unroll
         for (int c = 0; c < D; ++c) uarg[k * D + c] = m_ext[k][c];
-      Prob::vf(uarg, par, f);
+      vf_at<Prob>(uarg, t_vf, par, f);
 #pragma unroll
       for (int c = 0; c < D; ++c) z[c] = m_ext[Q][c] - f[c];
 #pragma unroll
@@ -1358,7 +1367,7 @@ __global__ void __launch_bounds__(THREADS * (1 + PAIR) + 64 * PIPE, (PIPE || PAI
       h[Q] = 1.0;
       if (D == 1 && Prob::HAS_JAC && a.correction == 1) {
         double J[Q * D * D];
-        Prob::jac(uarg, par, J);
+        jac_at<Prob>(uarg, t_vf, par, J);
 #pragma unroll
         for (int k = 0; k < Q; ++k) h[k] = -J[k];
       }

@@ -4,6 +4,9 @@
 // A user writes the vector field once, templated on the number type:
 //   template <class T> PN_DEV void vf(const T* u, const double* p, T* f)     u = (u, u', ...)[Q*D] -> f[D]
 // and optionally  PN_DEV void jac(const double* u, const double* p, double* J)   J[D][Q*D].
+// A time-dependent field (registered with PN_B200_FORM_TIME_DEPENDENT) takes the time after the state:
+//   template <class T> PN_DEV void vf(const T* u, const T& t, const double* p, T* f)
+//   PN_DEV void jac(const double* u, double t, const double* p, double* J)
 // UserProblem evaluates it on doubles for the step, on truncated Taylor series (Jet<N>) for the Taylor-mode
 // initialisation, and -- when the user gives no Jacobian -- on Jet<2> once per state column for the Jacobian.
 //
@@ -304,16 +307,31 @@ using jet::Jet;
 
 // Problem functor over a user source `Src` with Src::vf<T> (and Src::jac when HAS_SRC_JAC): the interface of the
 // functors in pn_problems.cuh.  ID is not read by any kernel; the registry keys user problems by their own id.
-template <class Src, int D_, int Q_, int P_, bool HAS_SRC_JAC>
+// TIME_: Src::vf<T>(u, t, p, f) and Src::jac(u, t, p, J) take the time, as a number of type T (a Jet<N> in the
+// Taylor-mode initialisation, the constant (t, 0) in the derived Jacobian); an autonomous source never sees it.
+template <class Src, int D_, int Q_, int P_, bool HAS_SRC_JAC, bool TIME_ = false>
 struct UserProblem {
   static constexpr int D = D_, Q = Q_, P = P_, ID = -1;
-  static constexpr bool HAS_JAC = true;
-  PN_DEV static void vf(const double* u, const double* par, double* f) { Src::template vf<double>(u, par, f); }
+  static constexpr bool HAS_JAC = true, TIME = TIME_;
+  template <class T>
+  PN_DEV static void src_vf(const T* u, const T& t, const double* par, T* f) {
+    if constexpr (TIME)
+      Src::template vf<T>(u, t, par, f);
+    else
+      Src::template vf<T>(u, par, f);
+  }
+  PN_DEV static void vf(const double* u, const double* par, double* f) { src_vf<double>(u, 0.0, par, f); }
+  PN_DEV static void vf(const double* u, double t, const double* par, double* f) { src_vf<double>(u, t, par, f); }
+  PN_DEV static void jac(const double* u, const double* par, double* J) { jac(u, 0.0, par, J); }
   // without a user Jacobian: column j is the first-order coefficient of vf at u + eps e_j
-  PN_DEV static void jac(const double* u, const double* par, double* J) {
+  PN_DEV static void jac(const double* u, double t, const double* par, double* J) {
     if constexpr (HAS_SRC_JAC) {
-      Src::jac(u, par, J);
+      if constexpr (TIME)
+        Src::jac(u, t, par, J);
+      else
+        Src::jac(u, par, J);
     } else {
+      const Jet<2> tj(t);
       for (int j = 0; j < Q * D; ++j) {
         Jet<2> x[Q * D], f[D];
 #pragma unroll
@@ -321,7 +339,7 @@ struct UserProblem {
           x[i].c[0] = u[i];
           x[i].c[1] = (i == j) ? 1.0 : 0.0;
         }
-        Src::template vf<Jet<2>>(x, par, f);
+        src_vf<Jet<2>>(x, tj, par, f);
 #pragma unroll
         for (int l = 0; l < D; ++l) J[l * Q * D + j] = f[l].c[1];
       }
@@ -329,12 +347,20 @@ struct UserProblem {
   }
   template <int N>
   PN_DEV static void vf_jet(const double* U, const double* par, double* F) {
-    Jet<N> x[Q * D], f[D];
+    vf_jet<N>(U, nullptr, par, F);
+  }
+  template <int N>
+  PN_DEV static void vf_jet(const double* U, const double* Tc, const double* par, double* F) {
+    Jet<N> x[Q * D], f[D], tj(0.0);
 #pragma unroll
     for (int i = 0; i < Q * D; ++i)
 #pragma unroll
       for (int k = 0; k < N; ++k) x[i].c[k] = U[i * N + k];
-    Src::template vf<Jet<N>>(x, par, f);
+    if constexpr (TIME) {
+#pragma unroll
+      for (int k = 0; k < N; ++k) tj.c[k] = Tc[k];
+    }
+    src_vf<Jet<N>>(x, tj, par, f);
 #pragma unroll
     for (int l = 0; l < D; ++l)
 #pragma unroll
@@ -342,17 +368,21 @@ struct UserProblem {
   }
 };
 
-// Problem functor over a user's `struct Problem` with the interface of pn_problems.cuh.  Its own Jacobian when it
-// has one, else column j is the first-order coefficient of vf_jet<2> at u + eps e_j.
+// Problem functor over a user's `struct Problem` with the interface of pn_problems.cuh (TIME included).  Its own
+// Jacobian when it has one, else column j is the first-order coefficient of vf_jet<2> at u + eps e_j, with the time
+// held constant.
 template <class Pr>
 struct FullProblem {
   static constexpr int D = Pr::D, Q = Pr::Q, P = Pr::P, ID = -1;
-  static constexpr bool HAS_JAC = true;
+  static constexpr bool HAS_JAC = true, TIME = TimeDependent<Pr>::value;
   PN_DEV static void vf(const double* u, const double* par, double* f) { Pr::vf(u, par, f); }
-  PN_DEV static void jac(const double* u, const double* par, double* J) {
+  PN_DEV static void vf(const double* u, double t, const double* par, double* f) { Pr::vf(u, t, par, f); }
+  PN_DEV static void jac(const double* u, const double* par, double* J) { jac(u, 0.0, par, J); }
+  PN_DEV static void jac(const double* u, double t, const double* par, double* J) {
     if constexpr (Pr::HAS_JAC) {
-      Pr::jac(u, par, J);
+      jac_at<Pr>(u, t, par, J);
     } else {
+      const double Tc[2] = {t, 0.0};
       for (int j = 0; j < Q * D; ++j) {
         double U[Q * D * 2], F[D * 2];
 #pragma unroll
@@ -360,7 +390,7 @@ struct FullProblem {
           U[2 * i] = u[i];
           U[2 * i + 1] = (i == j) ? 1.0 : 0.0;
         }
-        Pr::template vf_jet<2>(U, par, F);
+        vf_jet<2>(U, Tc, par, F);
 #pragma unroll
         for (int l = 0; l < D; ++l) J[l * Q * D + j] = F[2 * l + 1];
       }
@@ -370,33 +400,42 @@ struct FullProblem {
   PN_DEV static void vf_jet(const double* U, const double* par, double* F) {
     Pr::template vf_jet<N>(U, par, F);
   }
+  template <int N>
+  PN_DEV static void vf_jet(const double* U, const double* Tc, const double* par, double* F) {
+    if constexpr (TIME)
+      Pr::template vf_jet<N>(U, Tc, par, F);
+    else
+      Pr::template vf_jet<N>(U, par, F);
+  }
 };
 
-// ---- evaluation of a problem for users and tests (pn_b200_problem_evaluate) -------------------------------------
-// per state b: f = vf(u0, p), tc = taylor_init (the Taylor coefficients u^(k)(t0), k = 0..NU), J = jac(u0, p)
+// ---- evaluation of a problem for users and tests (pn_b200_problem_evaluate[_at]) ---------------------------------
+// per state b, at the time t0 = t[b] (0 without t): f = vf(u0, t0, p), tc = taylor_init (the Taylor coefficients
+// u^(k)(t0), k = 0..NU), J = jac(u0, t0, p)
 template <class Prob, int NU>
-__global__ void __launch_bounds__(128) pn_problem_eval_kernel(long long n, int num_params, const double* u0, const double* params,
-                                                              double* f, double* tc, double* J) {
+__global__ void __launch_bounds__(128) pn_problem_eval_kernel(long long n, int num_params, const double* t, const double* u0,
+                                                              const double* params, double* f, double* tc, double* J) {
   constexpr int D = Prob::D, Q = Prob::Q, P = (Prob::P > 0 ? Prob::P : 1);
   const long long b = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= n) return;
   double u[Q * D], par[P];
   for (int i = 0; i < Q * D; ++i) u[i] = u0[b * Q * D + i];
   for (int i = 0; i < P; ++i) par[i] = (i < num_params) ? params[b * num_params + i] : 0.0;
+  const double t0 = t ? t[b] : 0.0;
   if (f) {
     double fb[D];
-    Prob::vf(u, par, fb);
+    vf_at<Prob>(u, t0, par, fb);
     for (int l = 0; l < D; ++l) f[b * D + l] = fb[l];
   }
   if (tc) {
-    double t[NU + 1][D];
-    taylor_init<Prob, NU>(u, par, t);
+    double c[NU + 1][D];
+    taylor_init<Prob, NU>(u, t0, par, c);
     for (int k = 0; k <= NU; ++k)
-      for (int l = 0; l < D; ++l) tc[(b * (NU + 1) + k) * D + l] = t[k][l];
+      for (int l = 0; l < D; ++l) tc[(b * (NU + 1) + k) * D + l] = c[k][l];
   }
   if (J && Prob::HAS_JAC) {
     double Jb[D * Q * D];
-    Prob::jac(u, par, Jb);
+    jac_at<Prob>(u, t0, par, Jb);
     for (int e = 0; e < D * Q * D; ++e) J[b * D * Q * D + e] = Jb[e];
   }
 }

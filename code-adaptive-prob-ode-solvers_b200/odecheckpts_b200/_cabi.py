@@ -23,6 +23,7 @@ PROBLEM_IDS = {
 }
 USER_PROBLEM_BASE = 1024  # ids of problems registered at run time (register_problem) start here
 SOURCE_FORMS = {"simple": 0, "full": 1}
+FORM_TIME_DEPENDENT = 2  # OR-ed into the form: the field takes the time (include/pn_b200.h)
 FACTORISATIONS = {"isotropic": 0, "blockdiag": 1, "dense": 2}
 CORRECTIONS = {"ts0": 0, "ts1": 1}
 STRATEGIES = {"filter": 0, "fixedpoint": 1}
@@ -100,6 +101,7 @@ EXPORTS = (
     "pn_b200_last_error",
     "pn_b200_register_problem",
     "pn_b200_problem_evaluate",
+    "pn_b200_problem_evaluate_at",
     "pn_b200_compile",
 )
 
@@ -152,6 +154,8 @@ def lib():
                                                C.POINTER(C.c_int32)]  # fmt: skip
         L.pn_b200_problem_evaluate.restype = C.c_int
         L.pn_b200_problem_evaluate.argtypes = [C.c_int32, C.c_int32, C.c_int64] + [vp] * 6
+        L.pn_b200_problem_evaluate_at.restype = C.c_int
+        L.pn_b200_problem_evaluate_at.argtypes = [C.c_int32, C.c_int32, C.c_int64] + [vp] * 7
         L.pn_b200_compile.restype = C.c_int
         L.pn_b200_compile.argtypes = [C.POINTER(Desc)]
         _lib = L
@@ -188,14 +192,16 @@ def output_sizes(desc):
     return {name: int(getattr(sz, name)) for name, _ in Sizes._fields_}
 
 
-def register_problem(name, source, *, d, ode_order=1, num_params=0, form="simple"):
+def register_problem(name, source, *, d, ode_order=1, num_params=0, form="simple", time_dependent=False):
     """Compile a user-defined vector field (CUDA C++ source, see include/pn_b200.h) and return its problem id.
-    A compile error raises ValueError with the compiler log."""
+    ``time_dependent``: the field's functions take the time after the state.  A compile error raises ValueError
+    with the compiler log."""
     if form not in SOURCE_FORMS:
         raise ValueError(f"form must be one of {sorted(SOURCE_FORMS)}")
+    code = SOURCE_FORMS[form] | (FORM_TIME_DEPENDENT if time_dependent else 0)
     pid = C.c_int32(-1)
-    check(lib().pn_b200_register_problem(name.encode(), source.encode(), SOURCE_FORMS[form], int(d), int(ode_order),
-                                         int(num_params), C.byref(pid)))  # fmt: skip
+    check(lib().pn_b200_register_problem(name.encode(), source.encode(), code, int(d), int(ode_order), int(num_params),
+                                         C.byref(pid)))  # fmt: skip
     return pid.value
 
 
@@ -204,15 +210,20 @@ def compile_kernels(desc):
     check(lib().pn_b200_compile(C.byref(desc)))
 
 
-def problem_evaluate_device(problem, nu, u0, params, *, d, ode_order, f=True, taylor=True, jac=True, stream=None):
-    """The functor of `problem` at n states u0 [n, ode_order, d] (torch CUDA float64): dict with f [n, d],
-    taylor [n, nu + 1, d] (the Taylor-mode initialisation) and jac [n, d, ode_order * d], as requested."""
+def problem_evaluate_device(problem, nu, u0, params, *, d, ode_order, f=True, taylor=True, jac=True, stream=None, t=None):
+    """The functor of `problem` at n states u0 [n, ode_order, d] (torch CUDA float64) and times t [n] (None: 0):
+    dict with f [n, d], taylor [n, nu + 1, d] (the Taylor-mode initialisation) and jac [n, d, ode_order * d], as
+    requested."""
     import torch
 
     dev = u0.device
     n = u0.shape[0]
     u0 = u0.to(torch.float64).contiguous()
     params = None if params is None else params.to(device=dev, dtype=torch.float64).contiguous()
+    if t is not None:
+        t = torch.as_tensor(t, dtype=torch.float64, device=dev).contiguous()
+        if t.shape != (n,):
+            raise ValueError(f"t must have shape ({n},), got {tuple(t.shape)}")
     f64 = dict(dtype=torch.float64, device=dev)
     out = {}
     if f:
@@ -227,8 +238,8 @@ def problem_evaluate_device(problem, nu, u0, params, *, d, ode_order, f=True, ta
 
     s = torch.cuda.current_stream(dev) if stream is None else stream
     with torch.cuda.device(dev):
-        rc = lib().pn_b200_problem_evaluate(int(problem), int(nu), int(n), ptr(u0), ptr(params), ptr(out.get("f")),
-                                            ptr(out.get("taylor")), ptr(out.get("jac")), C.c_void_p(s.cuda_stream))  # fmt: skip
+        rc = lib().pn_b200_problem_evaluate_at(int(problem), int(nu), int(n), ptr(t), ptr(u0), ptr(params), ptr(out.get("f")),
+                                               ptr(out.get("taylor")), ptr(out.get("jac")), C.c_void_p(s.cuda_stream))  # fmt: skip
     check(rc)
     return out
 

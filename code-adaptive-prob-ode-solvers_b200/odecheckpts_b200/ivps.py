@@ -30,12 +30,13 @@ class _Tracer:
 
 
 class VectorField:
-    def __init__(self, name, d, ode_order, num_params, fun, problem_id=None):
+    def __init__(self, name, d, ode_order, num_params, fun, problem_id=None, time_dependent=False):
         self.name = name
         self.problem_id = PROBLEM_IDS[name] if problem_id is None else problem_id
         self.d = d
         self.ode_order = ode_order
         self.num_params = num_params
+        self.time_dependent = time_dependent
         self._fun = fun
 
     def __call__(self, *u, t=None, p=()):
@@ -46,7 +47,10 @@ class VectorField:
             return _Tracer(u[0].shape)
         if self._fun is None:
             raise TypeError(f"{self.name}: no host function was given (cuda_vector_field(..., host=...))")
-        return self._fun(*[np.asarray(x, dtype=np.float64) for x in u], *_flat_params(p))
+        args = [np.asarray(x, dtype=np.float64) for x in u] + _flat_params(p)
+        if self.time_dependent:
+            return self._fun(*args, t=t)
+        return self._fun(*args)
 
     def __repr__(self):
         return f"VectorField({self.name!r}, d={self.d}, ode_order={self.ode_order})"
@@ -83,7 +87,7 @@ def resolve_vector_field(vf, u0, t0=0.0):
     return records[0]
 
 
-def cuda_vector_field(name, source, *, d, ode_order=1, num_params=0, form="simple", host=None):
+def cuda_vector_field(name, source, *, d, ode_order=1, num_params=0, form="simple", host=None, time_dependent=False):
     """A user-defined vector field, compiled at run time into the solver kernels.
 
     ``source`` is CUDA C++.  ``form="simple"``: one function templated on the number type,
@@ -97,10 +101,17 @@ def cuda_vector_field(name, source, *, d, ode_order=1, num_params=0, form="simpl
     interface of the built-in functors (csrc/pn_problems.cuh).  Compile errors raise ValueError with
     the compiler log; its line numbers are the lines of ``source``.
 
-    ``host`` is an optional numpy function ``host(*u, *params)`` kept for truth solutions; it is
-    what the returned VectorField evaluates when called with arrays."""
-    pid = _cabi.register_problem(name, source, d=d, ode_order=ode_order, num_params=num_params, form=form)
-    return VectorField(name, d, ode_order, num_params, host, problem_id=pid)
+    ``time_dependent=True`` registers a non-autonomous field: the functions take the time after the
+    state, ``vf(const T* u, const T& t, const double* p, T* f)`` and ``jac(u, double t, p, J)``
+    (``form="full"``: ``TIME = true``, ``vf(u, t, p, f)``, ``jac(u, t, p, J)``, ``vf_jet<N>(U, Tc, p, F)``).
+    The solver evaluates the field at the time the step or checkpoint it attempts commits.
+
+    ``host`` is an optional numpy function ``host(*u, *params)`` (``host(*u, *params, t=t)`` for a
+    time-dependent field) kept for truth solutions; it is what the returned VectorField evaluates
+    when called with arrays."""
+    pid = _cabi.register_problem(name, source, d=d, ode_order=ode_order, num_params=num_params, form=form,
+                                 time_dependent=time_dependent)  # fmt: skip
+    return VectorField(name, d, ode_order, num_params, host, problem_id=pid, time_dependent=time_dependent)
 
 
 # ---- the zoo ---------------------------------------------------------------------------------

@@ -194,6 +194,17 @@ int pn_b200_get_last_timing(float* solve_ms, float* smooth_ms);
  *                        with J[d][ode_order * d]; without it the Jacobian is derived from vf on pn::Jet<2>.
  *   PN_B200_FORM_FULL    struct Problem with the interface of the built-in functors (csrc/pn_problems.cuh):
  *                        D, Q, P, HAS_JAC, vf, jac, vf_jet<N>.
+ * OR-ed into `form`, PN_B200_FORM_TIME_DEPENDENT registers a non-autonomous field, whose functions take the time
+ * after the state:
+ *   simple               template <class T> PN_DEV void vf(const T* u, const T& t, const double* p, T* f), and
+ *                        optionally  PN_DEV void jac(const double* u, double t, const double* p, double* J).  In the
+ *                        Taylor-mode initialisation t is the series (t0, 1, 0, ...), so the coefficients are the
+ *                        exact derivatives u^(k)(t0).
+ *   full                 struct Problem with  static constexpr bool TIME = true,  vf(u, t, p, f), jac(u, t, p, J)
+ *                        and vf_jet<N>(U, Tc, p, F), Tc[N] the time's normalised Taylor coefficients.
+ * The solver evaluates the field (and the Jacobian) of an attempted step at its end, t + dt, or at the checkpoint
+ * it is aimed at: the time the step commits when it is accepted.  The flag is part of the registration: the same
+ * name and source with and without it are two problems.
  * Registration compiles a check kernel: a compile error returns PN_B200_ERR_ARGUMENT, and pn_b200_last_error()
  * holds the whole compiler log, whose line numbers are the lines of `source` under the file name `name`
  * ([A-Za-z0-9_.-], at most 128 characters).  Registering the same (name, source, form, sizes) again returns the
@@ -209,7 +220,7 @@ int pn_b200_get_last_timing(float* solve_ms, float* smooth_ms);
  * dense register-column kernel ((nu + 1) d <= 32).
  */
 enum { PN_B200_USER_PROBLEM_BASE = 1024 };
-enum { PN_B200_FORM_SIMPLE = 0, PN_B200_FORM_FULL = 1 };
+enum { PN_B200_FORM_SIMPLE = 0, PN_B200_FORM_FULL = 1, PN_B200_FORM_TIME_DEPENDENT = 2 };
 int pn_b200_register_problem(const char* name, const char* source, int form, int32_t d, int32_t ode_order,
                              int32_t num_params, int32_t* problem_id);
 
@@ -228,6 +239,10 @@ int pn_b200_compile(const pn_b200_desc* desc);
  */
 int pn_b200_problem_evaluate(int32_t problem, int32_t nu, int64_t n, const double* u0, const double* params, double* f,
                              double* taylor, double* jac, void* cuda_stream);
+/* The same at per-state times t [n] (DEVICE; NULL: 0), for time-dependent problems: f and jac at (t, u0), taylor the
+ * coefficients u^(k)(t).  An autonomous problem ignores t. */
+int pn_b200_problem_evaluate_at(int32_t problem, int32_t nu, int64_t n, const double* t, const double* u0,
+                                const double* params, double* f, double* taylor, double* jac, void* cuda_stream);
 
 /* Human-readable description of the last error on the calling thread. */
 const char* pn_b200_last_error(void);

@@ -11,6 +11,13 @@ resident on the device):
   simple   the formula templated on the number type (form "simple"), Taylor coefficients and Jacobian derived
 Reports solves/s, registers and stack per thread of the solve kernel, whether the outputs are bit-identical to the
 built-in's, and the NVRTC compile time of one module of each kernel family.
+
+Time-dependent fields, on the same workload:
+  simple-t  the simple-form formula registered time-dependent, vf(u, t, p, f) ignoring t, against `simple` (the same
+            formula registered autonomous): the cost of passing the time, in registers, stack and time (alternating
+            rounds)
+  forced    forced Van der Pol, x'' = mu ((1 - x^2) x' - x) + A cos(w t), A = 1e3, with a forcing frequency w per
+            member in [0.5, 2]: time per ensemble and attempted steps
 """
 
 import argparse
@@ -37,6 +44,10 @@ FULL = """struct Problem {
   template <int N> PN_DEV static void vf_jet(const double* U, const double* p, double* F) { pn::VanDerPol::vf_jet<N>(U, p, F); }
 };"""
 SIMPLE = "template <class T> PN_DEV void vf(const T* u, const double* p, T* f) { f[0] = p[0] * fma(u[1], fma(-u[0], u[0], 1.0), -u[0]); }"
+SIMPLE_T = "template <class T> PN_DEV void vf(const T* u, const T& t, const double* p, T* f) { f[0] = p[0] * fma(u[1], fma(-u[0], u[0], 1.0), -u[0]); }"
+FORCED = """template <class T> PN_DEV void vf(const T* u, const T& t, const double* p, T* f) {
+  f[0] = fma(p[0], fma(u[1], fma(-u[0], u[0], 1.0), -u[0]), p[1] * cos(p[2] * t));
+}"""
 LORENZ96 = """template <class T> PN_DEV void vf(const T* u, const double* p, T* f) {
   for (int i = 0; i < 8; ++i) f[i] = (u[(i + 1) % 8] - u[(i + 6) % 8]) * u[(i + 7) % 8] - u[i] + p[0];
 }"""
@@ -47,15 +58,32 @@ LORENZ63 = """template <class T> PN_DEV void vf(const T* u, const double* p, T* 
 }"""
 
 
-def headline_desc(problem, B):
+def headline_desc(problem, B, P=1):
     return C.Desc(problem, 1, bench.NU, 2, C.FACTORISATIONS["dense"], C.CORRECTIONS["ts1"], C.STRATEGIES["fixedpoint"],
                   C.CALIBRATIONS["dynamic"], bench.TOL, bench.TOL, 0.01, 0.95, 0.2, 10.0, 0.3, 0.4, B, bench.K_CHECKPOINTS,
-                  0, 1, 0, 0)  # fmt: skip
+                  0, P, 0, 0)  # fmt: skip
 
 
 def desc_for(problem, d, nu, fact, corr, strat, B, P):
     return C.Desc(problem, d, nu, 1, C.FACTORISATIONS[fact], C.CORRECTIONS[corr], C.STRATEGIES[strat], C.CALIBRATIONS["dynamic"],
                   1e-6, 1e-6, 0.01, 0.95, 0.2, 10.0, 0.3, 0.4, B, 20, 0, P, 0, 0)  # fmt: skip
+
+
+def alternate(descs, inputs, ws, outs, rounds):
+    """ms per launch of each desc (CUDA events around solve + smoothing), rounds in rotating order"""
+    times = {k: [] for k in descs}
+    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    order = list(descs)
+    for r in range(rounds):
+        s = r % len(order)
+        for k in order[s:] + order[:s]:  # rotate who goes first
+            u0_d, par_d, save_d = inputs[k]
+            ev0.record()
+            C.solve_device(descs[k], u0_d, par_d, None, save_d, None, workspace=ws[k], out=outs[k])
+            ev1.record()
+            ev1.synchronize()
+            times[k].append(ev0.elapsed_time(ev1))
+    return {k: np.array(v) for k, v in times.items()}
 
 
 def timed_compile(desc):
@@ -132,22 +160,47 @@ def main():
         same = all(np.array_equal(outs[k][key].cpu().numpy(), ref[key]) for key in bench.DUMP_KEYS)
         say(f"  {k:8s} outputs (u, u_std, counters, status) bit-identical to the built-in's: {same}")
 
-    times = {k: [] for k in descs}
-    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    order = list(descs)
-    for r in range(args.rounds):
-        for k in order[r % 3:] + order[: r % 3]:  # rotate who goes first
-            ev0.record()
-            C.solve_device(descs[k], u0_d, par_d, None, save_d, None, workspace=ws[k], out=outs[k])
-            ev1.record()
-            ev1.synchronize()
-            times[k].append(ev0.elapsed_time(ev1))
+    times = alternate(descs, {k: (u0_d, par_d, save_d) for k in descs}, ws, outs, args.rounds)
     say(f"\nsolve + smoothing, CUDA events, {args.rounds} rounds in rotating order (ms per launch):")
     base = np.median(times["builtin"])
     for k, ts in times.items():
-        ts = np.array(ts)
         say(f"  {k:8s} median {np.median(ts):8.2f}  min {ts.min():8.2f}  max {ts.max():8.2f}   "
             f"{B / np.median(ts) * 1e3:12.0f} solves/s   {np.median(ts) / base:6.3f}x built-in")  # fmt: skip
+
+    # ---- time-dependent fields ----
+    say("\n## time-dependent fields on the headline workload")
+    t = time.perf_counter()
+    ids_t = {"simple": ids["simple"], "simple-t": C.register_problem("vdp_simple", SIMPLE_T, d=1, ode_order=2, num_params=1, time_dependent=True),
+             "forced": C.register_problem("vdp_forced", FORCED, d=1, ode_order=2, num_params=3, time_dependent=True)}  # fmt: skip
+    descs_t = {k: headline_desc(v, B, P=3 if k == "forced" else 1) for k, v in ids_t.items()}
+    for k in ("simple-t", "forced"):
+        C.compile_kernels(descs_t[k])
+    say(f"registration + compilation of the two time-dependent fields: {time.perf_counter() - t:.2f} s")
+    rng = np.random.default_rng(1)
+    par_f = np.stack([par[:, 0], np.full(B, 1e3), rng.uniform(0.5, 2.0, B)], 1)
+    inputs = {"simple": (u0_d, par_d, save_d), "simple-t": (u0_d, par_d, save_d), "forced": (u0_d, t64(par_f), save_d)}
+    outs_t, ws_t = {}, {}
+    for k, desc in descs_t.items():
+        o = C.solve_device(desc, *inputs[k][:2], None, save_d, None)
+        ws_t[k] = o["_workspace"]
+        outs_t[k] = {key: o[key] for key in bench.DUMP_KEYS}
+    torch.cuda.synchronize()
+    say("kernel info of the solve kernel:")
+    for k, desc in descs_t.items():
+        info = C.kernel_info(desc)
+        say(f"  {k:8s} registers {info['registers_per_thread']:3d}  stack {info['local_bytes_per_thread']:4d} B  "
+            f"ctas/SM {info['ctas_per_sm']}  grid {info['grid']}")  # fmt: skip
+    same = all(np.array_equal(outs_t["simple-t"][key].cpu().numpy(), outs_t["simple"][key].cpu().numpy()) for key in bench.DUMP_KEYS)
+    say(f"  simple-t outputs (u, u_std, counters, status) bit-identical to simple's: {same}")
+    times = alternate(descs_t, inputs, ws_t, outs_t, args.rounds)
+    say(f"\nsolve + smoothing, CUDA events, {args.rounds} rounds in rotating order (ms per launch):")
+    base = np.median(times["simple"])
+    for k, ts in times.items():
+        o = {key: v.cpu().numpy() for key, v in outs_t[k].items()}
+        att = (o["n_accepted"].reshape(B, -1)[:, -1] + o["n_rejected"].reshape(B, -1)[:, -1]).astype(np.int64)
+        say(f"  {k:8s} median {np.median(ts):8.2f}  min {ts.min():8.2f}  max {ts.max():8.2f}   {np.median(ts) / base:6.3f}x simple   "
+            f"attempted steps {att.sum():11d} (per member median {int(np.median(att))}, max {att.max()})  "
+            f"status != 0: {int((o['status'] != 0).sum())}")  # fmt: skip
     if args.out:
         os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
         with open(args.out, "w") as f:
