@@ -258,9 +258,15 @@ static int resolve(const pn_b200_desc* d, const KernelEntry** out) {
       }
     }
   }
-  if (k && (d->flags & PN_B200_FLAG_RECORD) && k->family != FAMILY_SCALAR && k->family != FAMILY_GROUP_ISO &&
-      k->family != FAMILY_GROUP_BDIAG && k->family != FAMILY_WIDE)
-    return fail(PN_B200_ERR_UNSUPPORTED, "trajectory recording is implemented for the thread-per-IVP, lane-per-dimension and CTA-per-IVP isotropic kernels");
+  // trajectory recording: the dense factorisation with d > 1 records in the register-column kernel (D <= 32) and the
+  // CTA-per-IVP dense kernel (the Brusselator's filter solves); the shared-memory dense kernel has no filter build
+  if ((d->flags & PN_B200_FLAG_RECORD) &&
+      ((k && k->family != FAMILY_SCALAR && k->family != FAMILY_GROUP_ISO && k->family != FAMILY_GROUP_BDIAG &&
+        k->family != FAMILY_WIDE && k->family != FAMILY_DENSE_ROWS && k->family != FAMILY_DENSE_CTA) ||
+       (!k && d->factorisation == PN_B200_DENSE && d->d > 1)))
+    return fail(PN_B200_ERR_UNSUPPORTED, "trajectory recording is implemented for the thread-per-IVP, lane-per-dimension and "
+                                         "CTA-per-IVP isotropic kernels and, for the dense factorisation with d > 1, the "
+                                         "register-column kernel ((nu+1) d <= 32) and the CTA-per-IVP dense kernel");
   if (!k) {
     char buf[256];
     snprintf(buf, sizeof buf, "no kernel compiled for problem=%d nu=%d factorisation=%d correction=%d strategy=%d d=%d",
@@ -457,7 +463,7 @@ int pn_b200_output_sizes(const pn_b200_desc* desc, pn_b200_sizes* sz) {
   sz->status = B;
   sz->traj_t = cap * B;
   sz->traj_u = cap * d * B;
-  sz->traj_std = cap * B;
+  sz->traj_std = cap * (dense ? d : 1) * B;
   sz->traj_len = rec ? B : 0;
   return PN_B200_SUCCESS;
 }

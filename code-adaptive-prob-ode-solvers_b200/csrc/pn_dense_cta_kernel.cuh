@@ -714,6 +714,17 @@ __global__ void __launch_bounds__(T, MINB) pn_dense_cta_kernel(const __grid_cons
     long long k_next = 1, n_acc = 0, n_rej = 0, n_att = 0;
     if (tid == 0) a.n_accepted[b * a.K] = 0;
     if (tid == 0 && a.out_scale) a.out_scale[b * a.K] = sigma0;
+    if constexpr (!FIX) {
+      // trajectory: traj_t [cap][B], traj_u and traj_std [cap][d][B]; thread l writes component l (and l + T, ...),
+      // thread 0 the time.  The initial point has a zero factor.
+      if (a.flags & FLAG_RECORD) {
+        if (tid == 0) a.traj_t[b] = t;
+        for (int l = tid; l < d; l += T) {
+          a.traj_u[(long long)l * a.B + b] = S_m[l];
+          a.traj_std[(long long)l * a.B + b] = 0.0;
+        }
+      }
+    }
     bool finished = false;
     int st = 0;
 
@@ -966,6 +977,20 @@ __global__ void __launch_bounds__(T, MINB) pn_dense_cta_kernel(const __grid_cons
         copy_vec(S_g, gm, Dn);
         copy_upper(S_LamU, M2, Dn);
       };
+      // filter: record the committed point (m_, U_ = L^T) as trajectory point n_acc.  The std of component l is
+      // sqrt((L L^T)_ll), the sum of squares of column l of U in ascending row order (the zeros below the diagonal
+      // add nothing); consecutive threads read consecutive columns
+      auto record = [&](double tt, const double* m_, const double* U_) {
+        if ((a.flags & FLAG_RECORD) && n_acc < a.traj_cap) {
+          if (tid == 0) a.traj_t[n_acc * a.B + b] = tt;
+          for (int l = tid; l < d; l += T) {
+            double acc = 0.0;
+            for (int j = 0; j <= l; ++j) acc = fma(U_[(size_t)j * Dn + l], U_[(size_t)j * Dn + l], acc);
+            a.traj_u[(n_acc * d + l) * a.B + b] = m_[l];
+            a.traj_std[(n_acc * d + l) * a.B + b] = dsqrt(acc);
+          }
+        }
+      };
       auto resolve_hits = [&]() {
         while (k_next < a.K && !(t + TIME_EPS < a.save_at[k_next])) {
           double* slot = slot_base + (size_t)k_next * SLOT;
@@ -1026,6 +1051,7 @@ __global__ void __launch_bounds__(T, MINB) pn_dense_cta_kernel(const __grid_cons
               copy_vec(S_m, m_new, Dn);
               copy_upper(S_U, Mc, Dn);
               if (FIX) commit_merged();
+              if constexpr (!FIX) record(t1, m_new, Mc);  // only the upper triangle of Mc is the factor
               resolve_hits();
             }
           } else {
@@ -1044,6 +1070,7 @@ __global__ void __launch_bounds__(T, MINB) pn_dense_cta_kernel(const __grid_cons
           set_identity();
         } else {
           emit_marg(slot, m_ext, U_ext);
+          if constexpr (!FIX) record(t_ck, m_ext, U_ext);
         }
         t = t_ck;
         copy_vec(S_m, m_ext, Dn);
@@ -1071,6 +1098,9 @@ __global__ void __launch_bounds__(T, MINB) pn_dense_cta_kernel(const __grid_cons
       a.status[b] = st;
       if (st != 0)
         for (long long kk = k_next; kk < a.K; ++kk) a.n_accepted[b * a.K + kk] = n_acc;
+      if constexpr (!FIX) {
+        if (a.flags & FLAG_RECORD) a.traj_len[b] = (n_acc + 1 < a.traj_cap) ? (n_acc + 1) : a.traj_cap;
+      }
     }
   }
 }

@@ -252,6 +252,17 @@ __global__ void __launch_bounds__(32 * WARPS) pn_dense_rows_kernel(const __grid_
         st = 0;
         if (c == 0) a.n_accepted[b * a.K] = 0;
         if (c == 0 && a.out_scale) a.out_scale[b * a.K] = sigma0;
+        if constexpr (!FIX) {
+          // trajectory: traj_t [cap][B], traj_u and traj_std [cap][d][B]; lane l < d writes component l, lane 0 the
+          // time.  The initial point has a zero factor.
+          if (a.flags & FLAG_RECORD) {
+            if (c == 0) a.traj_t[b] = t;
+            if (c < d) {
+              a.traj_u[(long long)c * a.B + b] = S_m[c];
+              a.traj_std[(long long)c * a.B + b] = 0.0;
+            }
+          }
+        }
       }
     }
     if (__all_sync(0xffffffffu, !have)) break;
@@ -669,6 +680,20 @@ __global__ void __launch_bounds__(32 * WARPS) pn_dense_rows_kernel(const __grid_
       for (int e = c; e < Dn; e += LANES) dst[e] = m_[e];
       for (int e = c; e < MAT; e += LANES) dst[Dn + e] = L_[e];
     };
+    // filter: record the committed point (m_, L_) as trajectory point n_acc.  Lane l < d owns row l of L_: the std
+    // of component l is sqrt((L L^T)_ll), its row's sum of squares in ascending order (the zeros right of the
+    // diagonal add nothing)
+    auto record = [&](double tt, const double* m_, const double* L_) {
+      if ((a.flags & FLAG_RECORD) && n_acc < a.traj_cap) {
+        if (c == 0) a.traj_t[n_acc * a.B + b] = tt;
+        if (c < d) {
+          double acc = 0.0;
+          for (int j = 0; j <= c; ++j) acc = fma(L_[c * Dn + j], L_[c * Dn + j], acc);
+          a.traj_u[(n_acc * d + c) * a.B + b] = m_[c];
+          a.traj_std[(n_acc * d + c) * a.B + b] = dsqrt(acc);
+        }
+      }
+    };
     auto resolve_hits = [&]() {
       while (k_next < a.K && !(t + TIME_EPS < a.save_at[k_next])) {
         double* slot = slot_base + (size_t)k_next * SLOT;
@@ -733,6 +758,7 @@ __global__ void __launch_bounds__(32 * WARPS) pn_dense_rows_kernel(const __grid_
               gcopy(S_g, gm, Dn);
               pack_lam();
             }
+            if constexpr (!FIX) record(t1, m_new, L_new);
             resolve_hits();
           }
         } else {
@@ -751,6 +777,7 @@ __global__ void __launch_bounds__(32 * WARPS) pn_dense_rows_kernel(const __grid_
         set_identity();
       } else {
         emit_marg(slot, m_ext, L_ext);
+        if constexpr (!FIX) record(t_ck, m_ext, L_ext);
       }
       t = t_ck;
       gcopy(S_m, m_ext, Dn);
@@ -777,6 +804,9 @@ __global__ void __launch_bounds__(32 * WARPS) pn_dense_rows_kernel(const __grid_
         a.status[b] = st;
         if (st != 0)
           for (long long kk = k_next; kk < a.K; ++kk) a.n_accepted[b * a.K + kk] = n_acc;
+      }
+      if constexpr (!FIX) {
+        if (c == 0 && (a.flags & FLAG_RECORD)) a.traj_len[b] = (n_acc + 1 < a.traj_cap) ? (n_acc + 1) : a.traj_cap;
       }
       have = false;
     }

@@ -320,6 +320,15 @@ def _chol_shape(desc):
     return (B, K, n, n)
 
 
+def _traj_std_shape(desc):
+    """traj_std: [cap, B], or [cap, d, B] for the dense factorisation with d > 1 (one std per dimension; the
+    size pn_b200_output_sizes reports)."""
+    cap, B, d = desc.traj_capacity, desc.batch, desc.d
+    if desc.factorisation == FACTORISATIONS["dense"] and d > 1:
+        return (cap, d, B)
+    return (cap, B)
+
+
 class _HostPool:
     """Recycled page-locked result buffers for the host entry point.
 
@@ -401,7 +410,7 @@ def solve_host(desc, u0, params, tol, save_at, output_scale0, *, full=False, dev
     cap = desc.traj_capacity
     tt = _host_empty((cap, B)) if rec else None
     tu = _host_empty((cap, d, B)) if rec else None
-    ts = _host_empty((cap, B)) if rec else None
+    ts = _host_empty(_traj_std_shape(desc)) if rec else None
     tl = _host_empty((B,), np.int64) if rec else None
     rc = lib().pn_b200_solve_save_at_host(
         C.byref(desc), _np_ptr(u0), _np_ptr(params), _np_ptr(tol), _np_ptr(save_at), _np_ptr(output_scale0),
@@ -454,7 +463,7 @@ def solve_device(desc, u0, params, tol, save_at, output_scale0, *, full=False, w
             cap = desc.traj_capacity
             out["traj_t"] = torch.empty((cap, B), **f64)
             out["traj_u"] = torch.empty((cap, d, B), **f64)
-            out["traj_std"] = torch.empty((cap, B), **f64)
+            out["traj_std"] = torch.empty(_traj_std_shape(desc), **f64)
             out["traj_len"] = torch.empty(B, dtype=torch.int64, device=dev)
     need = workspace_bytes(desc)
     if workspace is None or workspace.numel() * workspace.element_size() < need:

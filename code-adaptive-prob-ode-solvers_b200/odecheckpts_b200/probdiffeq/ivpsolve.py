@@ -262,19 +262,25 @@ def solve_adaptive_save_every_step(vf, initial_condition, t0, t1, adaptive_solve
     Filter strategy: the recorded filter solution (what vdp.py uses).  Smoother strategy
     (src/odecheckpts/ivpsolvers.py:133-142): the smoothed solution at every accepted grid point plus the
     per-step backward conditionals (see _solve_smoother_every_step).  Unbatched results are trimmed to the
-    accepted grid; ensembles (filter only) return padded arrays plus `num_steps`."""
+    accepted grid; ensembles (filter only) return padded arrays plus `num_steps`.  With the dense factorisation and d > 1,
+    `u_std` is per dimension: [n, d] unbatched, [cap, d, B] for ensembles; the other factorisations record one std
+    for all dimensions."""
     if adaptive_solver.solver.strategy.name == "smoother":
         return _solve_smoother_every_step(vf, initial_condition, t0, t1, adaptive_solver, dt0, factorisation, max_steps, device)
     desc, out, _, batched = _solve(vf, initial_condition, np.asarray([t0, t1], dtype=np.float64), adaptive_solver, dt0,
                                    factorisation=factorisation, return_marginals=False, tol=None, max_attempts=0,
                                    device=device, flags=_cabi.FLAG_RECORD, traj_capacity=int(max_steps))  # fmt: skip
     tt, tu, ts, tl = out["traj_t"], out["traj_u"], out["traj_std"], out["traj_len"]
+    per_dim = ts.ndim == 3  # dense with d > 1: one std per dimension, [cap, d, B]
     if not batched:
         n = int(tl[0])
         if n >= max_steps:
             raise RuntimeError(f"more than max_steps={max_steps} accepted steps; raise max_steps")
         u = tu[:n, :, 0]
-        std = ts[:n, 0][:, None] * (np.ones((1, desc.d)) if not _is_torch(ts) else 1.0)
+        if per_dim:
+            std = ts[:n, :, 0]
+        else:
+            std = ts[:n, 0][:, None] * (np.ones((1, desc.d)) if not _is_torch(ts) else 1.0)
         return Solution(t=tt[:n, 0], u=u, u_std=std, output_scale=None, marginals=None, posterior=None,
                         num_steps=n - 1, num_rejected=out["n_rejected"][0], status=out["status"][0])  # fmt: skip
     return Solution(t=tt, u=tu, u_std=ts, output_scale=None, marginals=None, posterior=None,

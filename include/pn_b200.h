@@ -116,8 +116,12 @@ int pn_b200_output_sizes(const pn_b200_desc* desc, pn_b200_sizes* sizes);
  *                 output_scale0); blockdiag: [B][K][d], one scale per dimension
  *   n_accepted    [B][K]        cumulative accepted steps when checkpoint k was emitted
  *   n_rejected    [B], status [B]
- *   traj_*        PN_B200_FLAG_RECORD only: traj_t [cap][B], traj_u [cap][d][B], traj_std [cap][B],
- *                 traj_len [B]; NULL otherwise
+ *   traj_*        PN_B200_FLAG_RECORD only (filter strategy): traj_t [cap][B], traj_u [cap][d][B],
+ *                 traj_std [cap][B] (one std for all dimensions), or [cap][d][B] for the dense
+ *                 factorisation with d > 1 (per dimension: sqrt of the diagonal of L L^T), traj_len [B];
+ *                 NULL otherwise.  Point 0 is t0 (std 0), then one point per accepted step; a step that
+ *                 crosses checkpoints is recorded at the last of them, so the last point is at
+ *                 save_at[K-1].  traj_len = min(accepted steps + 1, cap): later points are dropped
  */
 int pn_b200_solve_save_at(const pn_b200_desc* desc, const double* u0, const double* params,
                           const double* tol, const double* save_at, const double* output_scale0,
