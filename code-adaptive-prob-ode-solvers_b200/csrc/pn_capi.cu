@@ -527,6 +527,7 @@ int pn_b200_solve_save_at(const pn_b200_desc* desc, const double* u0, const doub
   a.params = params;
   a.tol = tol;
   a.save_at = save_at;
+  a.save_stride = (desc->flags & PN_B200_FLAG_MEMBER_GRIDS) ? desc->num_save_at : 0;
   a.sigma0 = output_scale0;
   a.ticket = (unsigned long long*)workspace;
   a.cond = (double*)((char*)workspace + p.ws_ticket);
@@ -716,6 +717,19 @@ int pn_b200_solve_save_at_host(const pn_b200_desc* desc, const double* u0, const
   int rc = pn_b200_output_sizes(desc, &sz);
   if (rc) return rc;
   if (desc->batch == 0) return PN_B200_SUCCESS;
+  // per-member grids arrive in host memory here, so their precondition is checked: every row strictly increasing
+  const bool member_grids = (desc->flags & PN_B200_FLAG_MEMBER_GRIDS) != 0;
+  const size_t rows = member_grids ? (size_t)desc->batch : 1, nk = (size_t)desc->num_save_at;
+  if (member_grids) {
+    if (!save_at) return fail(PN_B200_ERR_ARGUMENT, "null required buffer");
+    for (size_t r = 0; r < rows; ++r)
+      for (size_t k = 1; k < nk; ++k)
+        if (!(save_at[r * nk + k] > save_at[r * nk + k - 1])) {
+          char buf[128];
+          snprintf(buf, sizeof buf, "save_at row %zu is not strictly increasing at index %zu", r, k);
+          return fail(PN_B200_ERR_ARGUMENT, buf);
+        }
+  }
   // the caller's current device is restored on every exit path
   struct DeviceGuard {
     int prev = -1;
@@ -741,7 +755,7 @@ int pn_b200_solve_save_at_host(const pn_b200_desc* desc, const double* u0, const
       {&d_u0, u0, nullptr, B * q * d * 8},
       {&d_par, P ? params : nullptr, nullptr, P ? B * P * 8 : 0},
       {&d_tol, tol, nullptr, tol ? B * 2 * 8 : 0},
-      {&d_save, save_at, nullptr, K * 8},
+      {&d_save, save_at, nullptr, rows * K * 8},
       {&d_os, output_scale0, nullptr, output_scale0 ? B * 8 : 0},
       {&d_u, nullptr, u, sz.u * 8},
       {&d_std, nullptr, u_std, sz.u_std * 8},

@@ -708,7 +708,7 @@ __global__ void __launch_bounds__(T, MINB) pn_dense_cta_kernel(const __grid_cons
       for (size_t e = tid; e < MAT; e += T) slot_base[Dn + e] = 0.0;
     }
     __syncthreads();
-    double t = a.save_at[0], dt_next = a.dt0, le_prev = 0.0;
+    double t = grid_row(a, b)[0], dt_next = a.dt0, le_prev = 0.0;
     double pend_t = 0.0, pend_sigma = 1.0, sigma_state = sigma0;
     int mode = MODE_STEP;
     long long k_next = 1, n_acc = 0, n_rej = 0, n_att = 0;
@@ -729,7 +729,7 @@ __global__ void __launch_bounds__(T, MINB) pn_dense_cta_kernel(const __grid_cons
     int st = 0;
 
     while (!finished) {
-      const double t_ck = a.save_at[k_next < a.K ? k_next : a.K - 1];
+      const double t_ck = grid_row(a, b)[k_next < a.K ? k_next : a.K - 1];
       double dt, sigma_given;
       if (mode == MODE_STEP) {
         dt = (a.flags & FLAG_FIXED_GRID) ? (t_ck - t) : dt_next;
@@ -992,7 +992,7 @@ __global__ void __launch_bounds__(T, MINB) pn_dense_cta_kernel(const __grid_cons
         }
       };
       auto resolve_hits = [&]() {
-        while (k_next < a.K && !(t + TIME_EPS < a.save_at[k_next])) {
+        while (k_next < a.K && !(t + TIME_EPS < grid_row(a, b)[k_next])) {
           double* slot = slot_base + (size_t)k_next * SLOT;
           __syncthreads();
           if (FIX) {
@@ -1013,7 +1013,7 @@ __global__ void __launch_bounds__(T, MINB) pn_dense_cta_kernel(const __grid_cons
         if (k_next >= a.K) finished = true;
       };
       auto after_checkpoint = [&]() {
-        if (k_next < a.K && pend_t > a.save_at[k_next] + TIME_EPS) {
+        if (k_next < a.K && pend_t > grid_row(a, b)[k_next] + TIME_EPS) {
           mode = MODE_INTERP_A;
         } else {
           t = pend_t;

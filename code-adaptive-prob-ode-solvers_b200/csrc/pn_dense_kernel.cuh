@@ -206,7 +206,7 @@ __global__ void __launch_bounds__(32 * WARPS) pn_dense_kernel(const __grid_const
       double u0[Q * d], tc[N][d];
 #pragma unroll
       for (int i = 0; i < Q * d; ++i) u0[i] = a.u0[b * (Q * d) + i];
-      taylor_init<Prob, NU>(u0, a.save_at[0], par, tc);
+      taylor_init<Prob, NU>(u0, grid_row(a, b)[0], par, tc);
       if (lane == 0) {
 #pragma unroll
         for (int i = 0; i < N; ++i)
@@ -222,7 +222,7 @@ __global__ void __launch_bounds__(32 * WARPS) pn_dense_kernel(const __grid_const
       for (int e = lane; e < Dn; e += 32) slot_base[e] = S_m[e];
       for (int e = lane; e < MAT; e += 32) slot_base[Dn + e] = 0.0;
     }
-    double t = a.save_at[0], dt_next = a.dt0, le_prev = 0.0;
+    double t = grid_row(a, b)[0], dt_next = a.dt0, le_prev = 0.0;
     double pend_t = 0.0, pend_sigma = 1.0, sigma_state = sigma0;
     int mode = MODE_STEP;
     long long k_next = 1, n_acc = 0, n_rej = 0, n_att = 0;
@@ -232,7 +232,7 @@ __global__ void __launch_bounds__(32 * WARPS) pn_dense_kernel(const __grid_const
     int st = 0;
 
     while (!finished) {
-      const double t_ck = a.save_at[k_next < a.K ? k_next : a.K - 1];
+      const double t_ck = grid_row(a, b)[k_next < a.K ? k_next : a.K - 1];
       double dt, sigma_given;
       if (mode == MODE_STEP) {
         dt = (a.flags & FLAG_FIXED_GRID) ? (t_ck - t) : dt_next;
@@ -501,7 +501,7 @@ __global__ void __launch_bounds__(32 * WARPS) pn_dense_kernel(const __grid_const
         for (int e = lane; e < MAT; e += 32) dst[Dn + e] = L_[e];
       };
       auto resolve_hits = [&]() {
-        while (k_next < a.K && !(t + TIME_EPS < a.save_at[k_next])) {
+        while (k_next < a.K && !(t + TIME_EPS < grid_row(a, b)[k_next])) {
           double* slot = slot_base + (size_t)k_next * SLOT;
           if (FIX) {
             emit_cond(slot, S_G, S_g, S_Lam);
@@ -521,7 +521,7 @@ __global__ void __launch_bounds__(32 * WARPS) pn_dense_kernel(const __grid_const
         if (k_next >= a.K) finished = true;
       };
       auto after_checkpoint = [&]() {
-        if (k_next < a.K && pend_t > a.save_at[k_next] + TIME_EPS) {
+        if (k_next < a.K && pend_t > grid_row(a, b)[k_next] + TIME_EPS) {
           mode = MODE_INTERP_A;
         } else {
           t = pend_t;

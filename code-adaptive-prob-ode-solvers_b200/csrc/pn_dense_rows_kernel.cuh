@@ -224,7 +224,7 @@ __global__ void __launch_bounds__(32 * WARPS) pn_dense_rows_kernel(const __grid_
           double u0[Q * d], tc[N][d];
 #pragma unroll
           for (int i = 0; i < Q * d; ++i) u0[i] = a.u0[b * (Q * d) + i];
-          taylor_init<Prob, NU>(u0, a.save_at[0], par, tc);
+          taylor_init<Prob, NU>(u0, grid_row(a, b)[0], par, tc);
           if (c == 0) {
 #pragma unroll
             for (int i = 0; i < N; ++i)
@@ -240,7 +240,7 @@ __global__ void __launch_bounds__(32 * WARPS) pn_dense_rows_kernel(const __grid_
           for (int e = c; e < Dn; e += LANES) slot_base[e] = S_m[e];
           for (int e = c; e < MAT; e += LANES) slot_base[Dn + e] = 0.0;
         }
-        t = a.save_at[0];
+        t = grid_row(a, b)[0];
         dt_next = a.dt0;
         le_prev = 0.0;
         pend_t = 0.0;
@@ -268,7 +268,7 @@ __global__ void __launch_bounds__(32 * WARPS) pn_dense_rows_kernel(const __grid_
     if (__all_sync(0xffffffffu, !have)) break;
     __syncwarp();
 
-    const double t_ck = a.save_at[k_next < a.K ? k_next : a.K - 1];
+    const double t_ck = grid_row(a, b)[k_next < a.K ? k_next : a.K - 1];
     double dt, sigma_given;
     if (mode == MODE_STEP) {
       dt = (a.flags & FLAG_FIXED_GRID) ? (t_ck - t) : dt_next;
@@ -695,7 +695,7 @@ __global__ void __launch_bounds__(32 * WARPS) pn_dense_rows_kernel(const __grid_
       }
     };
     auto resolve_hits = [&]() {
-      while (k_next < a.K && !(t + TIME_EPS < a.save_at[k_next])) {
+      while (k_next < a.K && !(t + TIME_EPS < grid_row(a, b)[k_next])) {
         double* slot = slot_base + (size_t)k_next * SLOT;
         if (FIX) {
           emit_running_cond(slot);
@@ -715,7 +715,7 @@ __global__ void __launch_bounds__(32 * WARPS) pn_dense_rows_kernel(const __grid_
       if (k_next >= a.K) finished = true;
     };
     auto after_checkpoint = [&]() {
-      if (k_next < a.K && pend_t > a.save_at[k_next] + TIME_EPS) {
+      if (k_next < a.K && pend_t > grid_row(a, b)[k_next] + TIME_EPS) {
         mode = MODE_INTERP_A;
       } else {
         t = pend_t;

@@ -51,7 +51,7 @@
 namespace pn {
 
 enum : int { MODE_STEP = 0, MODE_INTERP_A = 1, MODE_INTERP_B = 2 };
-enum : int { FLAG_FIXED_GRID = 1, FLAG_RECORD = 2 };
+enum : int { FLAG_FIXED_GRID = 1, FLAG_RECORD = 2, FLAG_MEMBER_GRIDS = 4 };
 
 struct SolveArgs {
   int32_t correction;   // 0 ts0, 1 ts1 (D == 1 only)
@@ -64,7 +64,7 @@ struct SolveArgs {
   const double* u0;       // [B][Q*D]
   const double* params;   // [B][P]
   const double* tol;      // nullable [B][2]
-  const double* save_at;  // [K]
+  const double* save_at;  // [K], or [B][K] (FLAG_MEMBER_GRIDS): read through grid_row()
   const double* sigma0;   // nullable [B]
   double* cond;           // workspace [B*dv][K][SLOT] (member-major: a lane's slot is contiguous, so its
                           // stores fill whole 32-byte sectors); slot 0 = terminal state
@@ -115,7 +115,15 @@ struct SolveArgs {
   // n x n, computed by the host (pn_capi.cu).  Kernel parameters live in the constant bank, so
   // DFMA reads these entries as immediate constant operands.
   double lq[100];
+  // row stride of save_at: 0 (one grid for all members) or K (FLAG_MEMBER_GRIDS).  Last, so that the fields above
+  // keep their parameter offsets.
+  long long save_stride;
 };
+
+// Member b's checkpoint grid, derived from b where it is read (member fetch, emitted checkpoints, the dense kernels), so
+// that no per-lane row pointer stays live through a step loop.  The step loop of pn_scalar_kernel reads the time of
+// checkpoint k_next from its shared-memory slot instead (ck_cached / set_ck).
+PN_DEV const double* grid_row(const SolveArgs& a, long long b) { return a.save_at + b * a.save_stride; }
 
 // ---- time-sliced scheduling: cold paths, kept out of line so that they do not disturb the register
 // allocation of the step -----------------------------------------------------------------------
@@ -254,7 +262,8 @@ static __device__ __noinline__ int slice_park_if_waiting(const SolveArgs* a, lon
 // the quantum grows to about an eighth of it (a finer one was measured slower: every hand-over stalls
 // the warp).  Evaluated at multiples of the base quantum only.
 static __device__ __noinline__ bool slice_quantum_reached(const SolveArgs& a, double t, long long n_att, long long b) {
-  const double t0 = a.save_at[0], t1 = a.save_at[a.K - 1];
+  const double* ts = grid_row(a, b);
+  const double t0 = ts[0], t1 = ts[a.K - 1];
   const double frac = fmax((t - t0) / (t1 - t0), 1e-3);
   const double target = 0.125 * (double)n_att / frac;
   long long q = a.slice_mask + 1;
@@ -291,7 +300,7 @@ struct Layout {
   static constexpr int NT = N * (N + 1) / 2;
   static constexpr int BW = N * N + N * D + NT;   // G (full), g, Lam (lower, packed)
   static constexpr int MARG = N * D + NT;         // mean, chol (lower, packed)
-  static constexpr int PEND = MARG + 2;           // + t1, sigma1
+  static constexpr int PEND = MARG + 3;           // + t1, sigma1, time of checkpoint k_next (see ck_cached)
   static constexpr int SLOT_FIX = BW + MARG;      // fixed-point slot: cond (+ terminal marginal in slot 0)
   static constexpr int SLOT_FILT = MARG;          // filter slot: the marginal itself
   __host__ __device__ static constexpr int tri(int i, int j) { return i * (i + 1) / 2 + j; }  // j <= i
@@ -904,20 +913,6 @@ __global__ void __launch_bounds__(THREADS * (1 + PAIR) + 64 * PIPE, (PIPE || PAI
   // iteration asked global memory for it twice, in the middle of the serial part of the step)
   long long pipe_ck_k = -1;
   double pipe_ck_t = 0.0;
-  auto ck_cached = [&](long long k) -> double {
-    const long long kc = k < a.K ? k : a.K - 1;
-    if constexpr (PIPE || PAIR) {
-      if (kc != pipe_ck_k) {
-        pipe_ck_k = kc;
-        pipe_ck_t = a.save_at[kc];
-      }
-      return pipe_ck_t;
-    } else {
-      // (reusing the time the head of the iteration has loaded for the bookkeeping's first look at the same
-      // checkpoint was measured on the headline workload: no gain, more spills)
-      return a.save_at[kc];
-    }
-  };
 #ifdef PN_PIPE_STATS
   long long pipe_tm = clock64();
 #define PN_MAIN_PHASE(w) do { if ((PIPE || PAIR) && tid == 0 && blockIdx.x == 0) { const long long now_ = clock64(); atomicAdd(a.ticket + (w), (unsigned long long)(now_ - pipe_tm)); pipe_tm = now_; } } while (0)
@@ -954,6 +949,7 @@ __global__ void __launch_bounds__(THREADS * (1 + PAIR) + 64 * PIPE, (PIPE || PAI
   const int tid = threadIdx.x;
 #define SBW(e) s_bw[(e) * THREADS + tid]
 #define SPEND(e) s_pend[(e) * THREADS + tid]
+#define SCK SPEND(Lay::PEND - 1)
 #define SM(i, c) s_state[((i) * D + (c)) * THREADS + tid]
 #define SL(i, j) s_state[(N * D + Lay::tri(i, j)) * THREADS + tid]
   constexpr int OFF_G = 0, OFF_g = N * N, OFF_LAM = N * N + N * D;
@@ -1015,6 +1011,24 @@ __global__ void __launch_bounds__(THREADS * (1 + PAIR) + 64 * PIPE, (PIPE || PAI
   double par[P];
   int mode = MODE_STEP;
   long long k_next = 1, n_acc = 0, n_rej = 0, n_att = 0;
+  // The time of checkpoint k_next (clamped to K - 1) in this member's grid.  PIPE / PAIR: cached in a register.
+  // Otherwise in the lane's shared-memory slot SCK, which set_ck() rewrites whenever k_next or the member changes:
+  // the step loop reads the slot and computes no row address (save_at + b * save_stride) of its own.
+  auto set_ck = [&]() {
+    if constexpr (!(PIPE || PAIR)) SCK = grid_row(a, b)[k_next < a.K ? k_next : a.K - 1];
+  };
+  auto ck_cached = [&]() -> double {
+    if constexpr (PIPE || PAIR) {
+      const long long kc = k_next < a.K ? k_next : a.K - 1;
+      if (kc != pipe_ck_k) {
+        pipe_ck_k = kc;
+        pipe_ck_t = grid_row(a, b)[kc];
+      }
+      return pipe_ck_t;
+    } else {
+      return SCK;
+    }
+  };
   double mle_ss = 0.0;  // solver_mle: sum over the accepted steps of z^T S^-1 z / d
   // utilisation statistics (per warp, flushed once at exit): loop iterations, lane-iterations with
   // work, lane-iterations spent on checkpoint interpolation
@@ -1140,7 +1154,7 @@ __global__ void __launch_bounds__(THREADS * (1 + PAIR) + 64 * PIPE, (PIPE || PAI
           for (int i = 0; i < N; ++i) SM(i, 0) = 0.0;  // dummy register column
         } else {
           double tc[N][DT];
-          taylor_init<Prob, NU>(u0, a.save_at[0], par, tc);
+          taylor_init<Prob, NU>(u0, grid_row(a, b)[0], par, tc);
 #pragma unroll
           for (int i = 0; i < N; ++i) {
             if constexpr (GROUP == 1) {
@@ -1165,13 +1179,15 @@ __global__ void __launch_bounds__(THREADS * (1 + PAIR) + 64 * PIPE, (PIPE || PAI
           for (int i = 0; i < N; ++i) SBW(OFF_G + i * N + i) = 1.0;
         }
         pair_reset = true;  // PAIR: the backward lane resets its running conditional in front of the next job
-        t = a.save_at[0];
+        t = grid_row(a, b)[0];
         dt_next = a.dt0;
         le_prev = 0.0;
         sigma_state = sigma0;
         mode = MODE_STEP;
         k_next = 1;
+        set_ck();
         pipe_reset = true;
+        pipe_ck_k = -1;  // the cached checkpoint time belongs to the previous member's grid
         n_acc = n_rej = n_att = 0;
         mle_ss = 0.0;
         if (leader) a.n_accepted[b * a.K] = 0;
@@ -1217,6 +1233,7 @@ __global__ void __launch_bounds__(THREADS * (1 + PAIR) + 64 * PIPE, (PIPE || PAI
           le_prev = io.le_prev;
           sigma_state = io.sigma_state;
           k_next = io.k_next;
+          set_ck();
           n_acc = io.n_acc;
           n_rej = io.n_rej;
           n_att = io.n_att;
@@ -1271,7 +1288,7 @@ __global__ void __launch_bounds__(THREADS * (1 + PAIR) + 64 * PIPE, (PIPE || PAI
     // need the whole warp -- and leave in front of the bookkeeping)
 
     // ---- choose this iteration's prediction --------------------------------------------
-    double t_ck = ck_cached(k_next);
+    double t_ck = ck_cached();
     double dt, sigma_given;
     if (mode == MODE_STEP) {
       dt = (a.flags & FLAG_FIXED_GRID) ? (t_ck - t) : dt_next;
@@ -1898,7 +1915,6 @@ __global__ void __launch_bounds__(THREADS * (1 + PAIR) + 64 * PIPE, (PIPE || PAI
         pipe_nops += 1;
       }
     };
-    auto ck_time = [&](long long k) { return ck_cached(k); };
     // wide mode, pass 3: everything the bookkeeping below does to the n x d mean arrays, in ONE
     // sweep over the owned columns (reads the old state, writes the new one).
     //   mw: what becomes the state mean   (0 keep, 1 m_new, 2 m_ext, 3 pending mean)
@@ -2113,7 +2129,7 @@ __global__ void __launch_bounds__(THREADS * (1 + PAIR) + 64 * PIPE, (PIPE || PAI
     };
     // exact hits on checkpoints by the committed state (m, L, running conditional): emit, reset
     auto resolve_hits = [&](bool& fin) {
-      while (k_next < a.K && !(t + TIME_EPS < ck_time(k_next))) {
+      while (k_next < a.K && !(t + TIME_EPS < ck_cached())) {
         double* slot = a.cond + ((long long)vb * a.K + k_next) * SLOT;
         if constexpr (WIDE) {
           double* ws = wcond + (size_t)k_next * wslot;
@@ -2150,6 +2166,7 @@ __global__ void __launch_bounds__(THREADS * (1 + PAIR) + 64 * PIPE, (PIPE || PAI
         if (leader) a.n_accepted[b * a.K + k_next] = n_acc;
         emit_scale(k_next, sigma_state);
         k_next += 1;
+        set_ck();
       }
       if (k_next >= a.K) fin = true;
     };
@@ -2162,7 +2179,7 @@ __global__ void __launch_bounds__(THREADS * (1 + PAIR) + 64 * PIPE, (PIPE || PAI
     // after a checkpoint was emitted while the accepted state waits in s_pend
     auto after_checkpoint = [&](bool& fin) {
       const double t1 = SPEND(0);
-      if (k_next < a.K && t1 > ck_time(k_next) + TIME_EPS) {
+      if (k_next < a.K && t1 > ck_cached() + TIME_EPS) {
         mode = MODE_INTERP_A;  // the next checkpoint lies inside the same step
       } else {
         commit_pending();
@@ -2269,6 +2286,7 @@ __global__ void __launch_bounds__(THREADS * (1 + PAIR) + 64 * PIPE, (PIPE || PAI
         mode = MODE_INTERP_B;
       } else {
         k_next += 1;
+        set_ck();
         after_checkpoint(finished);
       }
     } else {
@@ -2279,7 +2297,7 @@ __global__ void __launch_bounds__(THREADS * (1 + PAIR) + 64 * PIPE, (PIPE || PAI
       if constexpr (WIDE) {
         const bool term = (k_next == a.K - 1);
         const double t1p = SPEND(0);
-        const bool again = (k_next + 1 < a.K) && (t1p > a.save_at[k_next + 1] + TIME_EPS);
+        const bool again = (k_next + 1 < a.K) && (t1p > grid_row(a, b)[k_next + 1] + TIME_EPS);
         if (term) {
           wide_store_factor(wcond, 0);
           wide_store_L1(wcond, 1);
@@ -2295,6 +2313,7 @@ __global__ void __launch_bounds__(THREADS * (1 + PAIR) + 64 * PIPE, (PIPE || PAI
         }
       }
       k_next += 1;
+      set_ck();
       after_checkpoint(finished);
     }
     if constexpr (PAIR) PN_MAIN_PHASE(19);  // bookkeeping
@@ -2340,6 +2359,7 @@ __global__ void __launch_bounds__(THREADS * (1 + PAIR) + 64 * PIPE, (PIPE || PAI
   if (stat_interp_iters) atomicAdd(a.ticket + 3, (unsigned long long)stat_interp_iters);
 #undef SBW
 #undef SPEND
+#undef SCK
 #undef SM
 #undef SL
   (void)sigma_state;

@@ -30,6 +30,7 @@ STRATEGIES = {"filter": 0, "fixedpoint": 1}
 CALIBRATIONS = {"none": 0, "dynamic": 1, "mle": 2}
 FLAG_FIXED_GRID = 1
 FLAG_RECORD = 2
+FLAG_MEMBER_GRIDS = 4  # save_at is [B, K]: one grid per ensemble member
 STATUS_OK, STATUS_NAN, STATUS_MAX_ATTEMPTS = 0, 1, 2
 
 
@@ -391,11 +392,27 @@ def _host_empty(shape, dtype=np.float64):
     return np.empty(shape, dtype=dtype)
 
 
+def _grid_desc(desc, save_at):
+    """`desc` for a grid of shape [K] (shared by all members), or a copy with FLAG_MEMBER_GRIDS set for a grid
+    of shape [B, K] (row b: member b's grid)."""
+    if save_at is None or save_at.ndim == 1:
+        if desc.flags & FLAG_MEMBER_GRIDS:
+            raise ValueError(f"FLAG_MEMBER_GRIDS needs save_at of shape ({desc.batch}, {desc.num_save_at})")
+        return desc
+    if tuple(save_at.shape) != (desc.batch, desc.num_save_at):
+        raise ValueError(f"save_at must have shape ({desc.num_save_at},) or ({desc.batch}, {desc.num_save_at}), "
+                         f"got {tuple(save_at.shape)}")  # fmt: skip
+    desc = Desc.from_buffer_copy(desc)
+    desc.flags |= FLAG_MEMBER_GRIDS
+    return desc
+
+
 def solve_host(desc, u0, params, tol, save_at, output_scale0, *, full=False, device=0):
-    """Host-buffer entry point (numpy in, numpy out)."""
+    """Host-buffer entry point (numpy in, numpy out).  save_at: [K], or [B, K] for one grid per member."""
     B, K, d, n = desc.batch, desc.num_save_at, desc.d, desc.nu + 1
     f64 = lambda a: None if a is None else np.ascontiguousarray(a, dtype=np.float64)  # noqa: E731
     u0, params, tol, save_at, output_scale0 = map(f64, (u0, params, tol, save_at, output_scale0))
+    desc = _grid_desc(desc, save_at)
     out = {
         "u": _host_empty((B, K, d)),
         "u_std": _host_empty((B, K, d)),
@@ -427,7 +444,8 @@ def solve_host(desc, u0, params, tol, save_at, output_scale0, *, full=False, dev
 
 
 def solve_device(desc, u0, params, tol, save_at, output_scale0, *, full=False, workspace=None, out=None, stream=None):
-    """Device-pointer entry point: torch CUDA tensors in, torch CUDA tensors out (asynchronous)."""
+    """Device-pointer entry point: torch CUDA tensors in, torch CUDA tensors out (asynchronous).  save_at: [K], or
+    [B, K] for one grid per member (each row strictly increasing: not checked here)."""
     import torch
 
     dev = u0.device
@@ -447,6 +465,7 @@ def solve_device(desc, u0, params, tol, save_at, output_scale0, *, full=False, w
     u0, params, tol, save_at, output_scale0 = (
         chk(x, nm) for x, nm in zip((u0, params, tol, save_at, output_scale0), ("u0", "params", "tol", "save_at", "output_scale0"))
     )
+    desc = _grid_desc(desc, save_at)
     if out is None:
         out = {
             "u": torch.empty((B, K, d), **f64),

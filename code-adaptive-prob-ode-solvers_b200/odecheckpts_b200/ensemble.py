@@ -29,6 +29,12 @@ def shard_indices(B, rank, world_size):
     return np.arange(rank, B, world_size)
 
 
+def shard_grid(save_at, rank, world_size):
+    """This rank's checkpoint grid: a grid shared by all members ([K]) as it is, and of a per-member grid ([B, K],
+    numpy or torch) the rows that go with the rank's members: rows r, r+G, r+2G, ..."""
+    return save_at if save_at.ndim == 1 else save_at[rank::world_size]
+
+
 def shard_sizes(B, world_size):
     return [(B - r + world_size - 1) // world_size for r in range(world_size)]
 

@@ -155,12 +155,18 @@ def _make_desc(field, nu, fact, solver, atol, rtol, control, dt0, B, K, flags=0,
 def _solve(vf, init, save_at, adaptive_solver, dt0, *, factorisation, return_marginals, tol, max_attempts, device,
            flags=0, traj_capacity=0, keep_conditionals=False):  # fmt: skip
     save_np = np.asarray(save_at.detach().cpu() if _is_torch(save_at) else save_at, dtype=np.float64)
-    if save_np.ndim != 1 or len(save_np) < 2 or not np.all(np.diff(save_np) > 0):
-        raise ValueError("save_at must be a strictly increasing 1-d grid with at least two points")
-    field, params, inits, nu, fact = _prepare(vf, init, float(save_np[0]), factorisation)
+    if save_np.ndim not in (1, 2) or save_np.shape[-1] < 2 or not np.all(np.diff(save_np, axis=-1) > 0):
+        raise ValueError("save_at must be a strictly increasing grid with at least two points: [K], or [B, K] with one "
+                         "row per ensemble member")  # fmt: skip
+    field, params, inits, nu, fact = _prepare(vf, init, float(save_np.flat[0]), factorisation)
     use_torch, B, batched, u0, par, tol, scale = _stack_members(inits, params, tol, init.output_scale, field.num_params)
+    if save_np.ndim == 2:
+        if not batched:
+            raise ValueError("a [B, K] grid gives every ensemble member its own grid; a single IVP takes save_at [K]")
+        if save_np.shape[0] != B:
+            raise ValueError(f"save_at has {save_np.shape[0]} rows for an ensemble of {B} members")
     desc = _make_desc(field, nu, fact, adaptive_solver.solver, adaptive_solver.atol, adaptive_solver.rtol,
-                      adaptive_solver.control, dt0, B, len(save_np), flags, traj_capacity, max_attempts)  # fmt: skip
+                      adaptive_solver.control, dt0, B, save_np.shape[-1], flags, traj_capacity, max_attempts)  # fmt: skip
     if use_torch or keep_conditionals:
         import torch
 
@@ -197,10 +203,22 @@ def _solution(out, t_out, batched, return_marginals):
     )  # fmt: skip
 
 
+def _span(t0, t1):
+    """The grid [t0, t1]: [2], or [B, 2] when t0 or t1 is given per ensemble member ([B])."""
+    t0, t1 = (np.asarray(x.detach().cpu() if _is_torch(x) else x, dtype=np.float64) for x in (t0, t1))
+    if t0.ndim == 0 and t1.ndim == 0:
+        return np.asarray([t0, t1])
+    if t0.ndim > 1 or t1.ndim > 1:
+        raise ValueError("t0 and t1 must be scalars or [B] arrays (one per ensemble member)")
+    return np.stack(np.broadcast_arrays(t0, t1), axis=1)
+
+
 def solve_adaptive_save_at(vf, initial_condition, save_at, adaptive_solver, dt0, *, factorisation=None,
                            return_marginals=True, tol=None, max_attempts=0, device=None, keep_conditionals=False):  # fmt: skip
     """Adaptive solve that returns the posterior at the checkpoints `save_at` with O(K) memory
-    (fixed-point smoother) -- the reference's hot path (ivpsolvers.py:71-77; SURVEY 3.2)."""
+    (fixed-point smoother) -- the reference's hot path (ivpsolvers.py:71-77; SURVEY 3.2).  For an ensemble,
+    save_at may be [B, K]: row b is member b's grid (its own t0, t1 and checkpoints; `Solution.t` is then
+    [B, K], and stats.log_marginal_likelihood observes data[b, k] at save_at[b, k])."""
     if keep_conditionals and not return_marginals:
         raise ValueError("keep_conditionals=True needs return_marginals=True (the posterior object carries the handle)")
     _, out, t_out, batched = _solve(vf, initial_condition, save_at, adaptive_solver, dt0, factorisation=factorisation,
@@ -211,8 +229,8 @@ def solve_adaptive_save_at(vf, initial_condition, save_at, adaptive_solver, dt0,
 
 def solve_adaptive_terminal_values(vf, initial_condition, t0, t1, adaptive_solver, dt0, *, factorisation=None,
                                    tol=None, max_attempts=0, device=None):  # fmt: skip
-    """run.py:82-90: the same loop with a single checkpoint at t1."""
-    sol = solve_adaptive_save_at(vf, initial_condition, np.asarray([t0, t1], dtype=np.float64), adaptive_solver, dt0,
+    """run.py:82-90: the same loop with a single checkpoint at t1.  For an ensemble, t0 and t1 may be [B]."""
+    sol = solve_adaptive_save_at(vf, initial_condition, _span(t0, t1), adaptive_solver, dt0,
                                  factorisation=factorisation, return_marginals=True, tol=tol,
                                  max_attempts=max_attempts, device=device)  # fmt: skip
     last = lambda x: x[..., -1, :] if x is not None else None  # noqa: E731
@@ -264,10 +282,10 @@ def solve_adaptive_save_every_step(vf, initial_condition, t0, t1, adaptive_solve
     per-step backward conditionals (see _solve_smoother_every_step).  Unbatched results are trimmed to the
     accepted grid; ensembles (filter only) return padded arrays plus `num_steps`.  With the dense factorisation and d > 1,
     `u_std` is per dimension: [n, d] unbatched, [cap, d, B] for ensembles; the other factorisations record one std
-    for all dimensions."""
+    for all dimensions.  For an ensemble (filter strategy), t0 and t1 may be [B]: member b's last point is at t1[b]."""
     if adaptive_solver.solver.strategy.name == "smoother":
         return _solve_smoother_every_step(vf, initial_condition, t0, t1, adaptive_solver, dt0, factorisation, max_steps, device)
-    desc, out, _, batched = _solve(vf, initial_condition, np.asarray([t0, t1], dtype=np.float64), adaptive_solver, dt0,
+    desc, out, _, batched = _solve(vf, initial_condition, _span(t0, t1), adaptive_solver, dt0,
                                    factorisation=factorisation, return_marginals=False, tol=None, max_attempts=0,
                                    device=device, flags=_cabi.FLAG_RECORD, traj_capacity=int(max_steps))  # fmt: skip
     tt, tu, ts, tl = out["traj_t"], out["traj_u"], out["traj_std"], out["traj_len"]
@@ -288,7 +306,8 @@ def solve_adaptive_save_every_step(vf, initial_condition, t0, t1, adaptive_solve
 
 
 def solve_fixed_grid(vf, initial_condition, grid, solver, *, factorisation=None, atol=1.0, rtol=1.0, device=None):
-    """vdp.py:88-91: the same step on a given grid, no error control."""
+    """vdp.py:88-91: the same step on a given grid, no error control.  For an ensemble, grid may be [B, K]: row b
+    is member b's grid."""
     asolver = AdaptiveSolver(solver, atol, rtol, control_proportional_integral())
     _, out, t_out, batched = _solve(vf, initial_condition, grid, asolver, 1.0, factorisation=factorisation,
                                     return_marginals=False, tol=None, max_attempts=0, device=device,

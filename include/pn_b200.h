@@ -51,7 +51,8 @@ enum {
 enum { PN_B200_OK = 0, PN_B200_NAN = 1, PN_B200_MAX_ATTEMPTS = 2 };  /* status[b] */
 enum {
   PN_B200_FLAG_FIXED_GRID = 1, /* solve_fixed_grid (vdp.py:88-91): steps = diff(save_at), no rejection */
-  PN_B200_FLAG_RECORD = 2      /* solve_adaptive_save_every_step (vdp.py:77-79): record accepted steps */
+  PN_B200_FLAG_RECORD = 2,     /* solve_adaptive_save_every_step (vdp.py:77-79): record accepted steps */
+  PN_B200_FLAG_MEMBER_GRIDS = 4 /* save_at is [B][K]: row b is member b's grid (jax.vmap over save_at / t0 / t1) */
 };
 
 /* return codes of the entry points */
@@ -101,7 +102,15 @@ int pn_b200_output_sizes(const pn_b200_desc* desc, pn_b200_sizes* sizes);
  *   u0            [B][q][d]     initial values (u, u', ...)
  *   params        [B][P]        vector-field parameters (may be NULL if P == 0)
  *   tol           [B][2] | NULL per-member (atol, rtol); NULL: desc->atol/rtol for all
- *   save_at       [K]           checkpoints, strictly increasing, save_at[0] = t0
+ *   save_at       [K]           checkpoints, strictly increasing, save_at[0] = t0 (a precondition: not checked)
+ *                 [B][K]        with PN_B200_FLAG_MEMBER_GRIDS: row-major, row b is member b's grid, each row
+ *                               strictly increasing (not checked), save_at[b][0] = t0 of member b; K is the same
+ *                               for every member.  Combined with PN_B200_FLAG_FIXED_GRID row b is member b's
+ *                               step grid; with PN_B200_FLAG_RECORD (K = 2) row b is [t0_b, t1_b] and the
+ *                               recording semantics below hold per member (the last point is at t1_b).  The flag
+ *                               changes no output size, no workspace size and no supported configuration;
+ *                               sampling and the likelihood take no times (they read the finished solve's
+ *                               workspace), so they need no per-member argument.
  *   output_scale0 [B] | NULL    initial output scale (ivpsolvers.py:55,68); NULL: 1.0
  *   u, u_std      [B][K][d]     smoothed checkpoint means / marginal standard deviations
  *   marg_mean     [B][K][n][d] | NULL   full marginal means (n = nu+1; for the dense factorisation this
@@ -121,7 +130,7 @@ int pn_b200_output_sizes(const pn_b200_desc* desc, pn_b200_sizes* sizes);
  *                 factorisation with d > 1 (per dimension: sqrt of the diagonal of L L^T), traj_len [B];
  *                 NULL otherwise.  Point 0 is t0 (std 0), then one point per accepted step; a step that
  *                 crosses checkpoints is recorded at the last of them, so the last point is at
- *                 save_at[K-1].  traj_len = min(accepted steps + 1, cap): later points are dropped
+ *                 save_at[K-1] (save_at[b][K-1] with PN_B200_FLAG_MEMBER_GRIDS).  traj_len = min(accepted steps + 1, cap): later points are dropped
  */
 int pn_b200_solve_save_at(const pn_b200_desc* desc, const double* u0, const double* params,
                           const double* tol, const double* save_at, const double* output_scale0,
@@ -133,7 +142,8 @@ int pn_b200_solve_save_at(const pn_b200_desc* desc, const double* u0, const doub
 /*
  * The same call with HOST buffers (what a CPU caller such as the reference's experiment
  * scripts holds): allocates device memory, copies in, solves, copies out, synchronises.
- * `device` is the CUDA device ordinal.
+ * `device` is the CUDA device ordinal.  With PN_B200_FLAG_MEMBER_GRIDS it copies B*K grid points
+ * and returns PN_B200_ERR_ARGUMENT when a row is not strictly increasing.
  */
 int pn_b200_solve_save_at_host(const pn_b200_desc* desc, const double* u0, const double* params,
                                const double* tol, const double* save_at, const double* output_scale0,
@@ -161,7 +171,7 @@ int pn_b200_markov_sample(const pn_b200_desc* desc, const void* workspace, size_
  * fixed-point solve: stats.log_marginal_likelihood(u, standard_deviation=, posterior=),
  * src/odecheckpts/train_util.py:22-24 (the parameter-inference loss, forward value only).
  * `workspace` / `status` are the buffers the solve call used.  data: [B][K][d] observed values of u
- * at save_at[0..K-1]; obs_std: [B][K] observation noise standard deviations (> 0); lml: [B] (all
+ * at save_at[0..K-1] (member b's row save_at[b][0..K-1] with PN_B200_FLAG_MEMBER_GRIDS); obs_std: [B][K] observation noise standard deviations (> 0); lml: [B] (all
  * DEVICE pointers).  lml[b] is the running mean over the K data points of
  * log p(y_k | y_{k+1}, ..., y_{K-1}) -- probdiffeq's reverse Kalman-filter estimator -- i.e. the joint
  * log density divided by K; NaN for failed members.  Isotropic and blockdiag factorisations of any dimension and the
